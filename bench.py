@@ -2,7 +2,7 @@
 """bench.py -- throughput of the IQ->PCM hot path on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload am|fm|wbfm|ssb|mixed]
-                    [--signal tone|noise] [--blocks T] [--impl reference] [--no-extras]
+                    [--signal tone|noise] [--blocks T] [--impl reference] [--no-extras] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic IQ: every channel
@@ -64,7 +64,38 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary per-mode lines")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true", help="tuning runs only: skip the end-to-end leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the PCM and per-channel sample counts of the last timed step "
+                         "as DIR/<name>.npy (float32 / float64, at most 64 MB in all: a seeded sample of channels when larger); "
+                         "needs --steps K > 0")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 arm computed")
+    if args.dump_outputs and args.steps <= 0:
+        # the engine's state carries from step to step: comparable dumps need the same number of steps
+        ap.error("--dump-outputs needs --steps K > 0")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, pcm, counts, suffix="", budget=DUMP_BYTES):
+    """The last timed step's results as a caller receives them from sdr_get_pcm: pcm [channels][samples] as float32
+    (int16 values, exact) and counts [channels] as float64. Above `budget` bytes a fixed, seeded sample of whole
+    channels is written, with their indices in channels.npy, so that two builds can be compared row for row."""
+    import numpy as np
+    n, samples = pcm.shape
+    rows = np.arange(n)
+    budget -= 4096  # the three .npy headers
+    if n * (samples * 4 + 16) > budget:
+        keep = budget // (samples * 4 + 16)
+        if keep < 1:
+            raise SystemExit("--dump-outputs: one channel's PCM alone exceeds this rank's %d bytes" % budget)
+        rows = np.sort(np.random.default_rng(0xD0).choice(n, size=keep, replace=False))
+        np.save(os.path.join(out_dir, "channels%s.npy" % suffix), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "pcm%s.npy" % suffix), pcm[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, "counts%s.npy" % suffix), counts[rows].astype(np.float64))
 
 
 def peaks():
@@ -247,8 +278,9 @@ def shard_parity(R, synth, workload, channels, first_channel, n_blocks, device_i
 
 
 def bench_one(torch, R, synth, workload, channels, n_blocks, steps, warmup, signal, device, rank, world,
-              dist, want_e2e=True, first_channel=None):
-    """Times `steps` passes of one workload on this rank. Returns a dict of local results."""
+              dist, want_e2e=True, first_channel=None, want_outputs=False):
+    """Times `steps` passes of one workload on this rank. Returns a dict of local results; with
+    want_outputs, res["outputs"] is (pcm, counts) of the last timed step."""
     first = rank * channels if first_channel is None else first_channel
     modes = synth.modes_for(workload, channels, first_channel=first)
     nbytes = n_blocks * BLOCK_BYTES
@@ -293,6 +325,8 @@ def bench_one(torch, R, synth, workload, channels, n_blocks, steps, warmup, sign
     e0, e1 = timed(steps)
     barrier()
     clocks = sampler.stop() if sampler else None
+    # read back before the clock soak below runs further steps on the same engine
+    outputs = eng.get_pcm() if want_outputs else None
     ms = e0.elapsed_time(e1)
     launches = eng.launch_count - l0
     redo = eng.debug_dc_redo_count()
@@ -308,7 +342,7 @@ def bench_one(torch, R, synth, workload, channels, n_blocks, steps, warmup, sign
             clocks["sampled"] = "1.5 s soak of the same launch right after the timed region (region too short)"
     res = {"ms_total": ms, "launches": launches, "clocks": clocks, "steps": steps,
            "samples_per_step": channels * nbytes // 2, "h2d": channels * nbytes,
-           "d2h": channels * (nbytes // 64) * 2, "dc_redo": redo}
+           "d2h": channels * (nbytes // 64) * 2, "dc_redo": redo, "outputs": outputs}
     eng.set_stream(0)
     eng.close()
 
@@ -460,14 +494,11 @@ def main():
         modes = synth.modes_for(workload, channels).numpy()
         vals = []
         desc = None
-        t_begin = time.time()
         n_steps = args.steps if args.steps > 0 else 5
         for i in range(args.warmup + n_steps):
             v, desc = run_cpu_reference(workload, modes, n_blocks, seconds_target=1.0, signal=args.signal)
             if i >= args.warmup:
                 vals.append(v)
-            if time.time() - t_begin > 150:
-                break
         value = float(np.mean(vals)) if vals else v
         desc["value"] = round(value, 3)
         line = {"impl": "reference", "metric": METRIC, "value": round(value, 3), "unit": "Msamples/s",
@@ -498,7 +529,11 @@ def main():
         print("note: --gpus %d but WORLD_SIZE %d; using WORLD_SIZE" % (args.gpus, world), file=sys.stderr)
 
     res = bench_one(torch, R, synth, workload, channels, n_blocks, args.steps, args.warmup, args.signal,
-                    device, rank, world, dist, want_e2e=not args.no_e2e)
+                    device, rank, world, dist, want_e2e=not args.no_e2e, want_outputs=bool(args.dump_outputs))
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        dump_outputs(args.dump_outputs, *res.pop("outputs"), suffix="_rank%d" % rank if world > 1 else "",
+                     budget=DUMP_BYTES // world)  # DUMP_BYTES for the whole job
     if args.no_e2e:
         res.update(e2e_ms_total=float("inf"), e2e_sync_ms_total=float("inf"), e2e_copy_ms_total=float("inf"),
                    e2e_steps=0, e2e_copy_steps=0, e2e_paths_agree=None)

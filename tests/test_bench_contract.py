@@ -48,3 +48,62 @@ def test_reference_arm_line(n_gpus, workload, total):
     cb = line["cpu_baseline"]
     assert cb["kind"] in ("reference", "port") and cb["cores"] >= 1 and cb["value"] == line["value"] and cb["sample"]
     assert line["e2e"] == {"value": line["value"], "unit": "Msamples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_dump_outputs_samples_whole_channels_within_the_budget(tmp_path):
+    import numpy as np
+    import bench
+    pcm = np.repeat(np.arange(-300, 300, dtype=np.int16)[:, None], 1024, axis=1)
+    counts = np.arange(600, dtype=np.uint32)
+    for d in ("a", "b"):
+        (tmp_path / d).mkdir()
+        bench.dump_outputs(str(tmp_path / d), pcm, counts, budget=1 << 20)
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 1 << 20
+    rows = np.load(tmp_path / "a" / "channels.npy")
+    got = np.load(tmp_path / "a" / "pcm.npy")
+    assert got.dtype == np.float32 and rows.dtype == np.float64 and 0 < rows.size < 600
+    assert np.array_equal(got, pcm[rows.astype(np.int64)]) and np.array_equal(np.load(tmp_path / "a" / "counts.npy"), rows)
+    for name in ("channels", "pcm", "counts"):  # the sample is fixed
+        assert np.array_equal(np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy")))
+    (tmp_path / "c").mkdir()
+    bench.dump_outputs(str(tmp_path / "c"), pcm[:200], counts[:200], budget=1 << 20)
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "c"), pcm, counts, budget=4096)
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", str(tmp_path / "d")],
+                       capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode != 0 and "--steps" in r.stderr and not (tmp_path / "d").exists()
+    assert sorted(f.name for f in (tmp_path / "c").iterdir()) == ["counts.npy", "pcm.npy"]
+    assert np.array_equal(np.load(tmp_path / "c" / "pcm.npy"), pcm[:200])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_last_timed_step(tmp_path):
+    """Two runs write the same arrays, and they are the PCM an engine returns after the same number of
+    calls on the same input: the untimed warm-up (at least 3) plus the --steps timed ones."""
+    import numpy as np
+    import torch
+    import bench
+    import rtlsdrdiags_b200 as R
+    from rtlsdrdiags_b200 import synth
+    steps, channels, blocks = 4, 40, 2
+    nbytes = blocks * bench.BLOCK_BYTES
+    args = ["--workload", "mixed", "--channels", str(channels), "--blocks", str(blocks), "--steps", str(steps),
+            "--warmup", "1", "--no-extras", "--no-cpu", "--no-e2e"]
+    for d in ("a", "b"):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args + ["--dump-outputs", str(tmp_path / d)],
+                           capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+    got = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in ("pcm", "counts")}
+    for n, a in got.items():
+        assert np.array_equal(a, np.load(tmp_path / "b" / (n + ".npy")))
+    modes = synth.modes_for("mixed", channels)
+    iq = synth.make_bank("tone", modes, nbytes, 0xB200, torch.device("cuda", 0))
+    e = R.Engine(channels, 0, nbytes)
+    e.set_modes(modes.numpy())
+    for _ in range(3 + steps):
+        e.accept_iq_device(iq)
+    pcm, counts = e.get_pcm()
+    e.close()
+    assert got["pcm"].dtype == np.float32 and np.array_equal(got["pcm"], pcm.astype(np.float32))
+    assert got["counts"].dtype == np.float64 and np.array_equal(got["counts"], counts)

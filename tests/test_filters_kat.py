@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 import _oracle as O
+import _pins
 
 L = O.oracle()
 have_ref = O.ref("radiodiags") is not None
@@ -123,9 +124,9 @@ def test_q15_clamp_is_per_tap_and_order_dependent():
     assert y[-1] == np.int16(acc >> 15) and y[-1] != 0
 
 
-@pytest.mark.skipif(not have_ref, reason="oracle/_ref not built")
 def test_building_blocks_match_compiled_reference_on_random_input():
     R = O.ref("radiodiags")
+    got, ref = [], []
     rng = np.random.default_rng(3)
     x = rng.integers(-32768, 32768, size=200000, dtype=np.int16)
     x[1000:1200] = 32767
@@ -134,35 +135,46 @@ def test_building_blocks_match_compiled_reference_on_random_input():
         # the float designs are not exported; compare through each library's own quantiser
         hq = O.q15_taps(fid).astype(f32) / f32(32768)
         hq = np.where(O.q15_taps(fid) == -32768, f32(1.0), hq).astype(f32)
-        d = R.ref_dec16_new(len(hq), O._ptr(hq, O._pf), M)
-        yr = np.zeros(len(x) // M + 1, dtype=np.int16)
-        n = R.ref_dec16_run(d, O._ptr(x, O._pi16), len(x), O._ptr(yr, O._pi16))
-        R.ref_dec16_free(d)
-        assert np.array_equal(yr[:n], dec16_oracle(hq, M, x)), "filter %d" % fid
+        got.append(dec16_oracle(hq, M, x))
+        if R:
+            d = R.ref_dec16_new(len(hq), O._ptr(hq, O._pf), M)
+            yr = np.zeros(len(x) // M + 1, dtype=np.int16)
+            n = R.ref_dec16_run(d, O._ptr(x, O._pi16), len(x), O._ptr(yr, O._pi16))
+            R.ref_dec16_free(d)
+            ref.append(yr[:n])
     xf = rng.standard_normal(5000).astype(f32)
-    f = R.ref_fir_new(8, O._ptr(TAPS, O._pf))
-    yr = np.zeros(5000, dtype=f32)
-    R.ref_fir_run(f, O._ptr(xf, O._pf), 5000, O._ptr(yr, O._pf))
-    R.ref_fir_free(f)
-    assert np.array_equal(yr, fir_oracle(TAPS, xf))
+    got.append(fir_oracle(TAPS, xf))
+    if R:
+        f = R.ref_fir_new(8, O._ptr(TAPS, O._pf))
+        yr = np.zeros(5000, dtype=f32)
+        R.ref_fir_run(f, O._ptr(xf, O._pf), 5000, O._ptr(yr, O._pf))
+        R.ref_fir_free(f)
+        ref.append(yr)
     for b, a in [([1, -1], [-0.95]), ([0.0253863, 0.0253863], [-0.9492274]), ([1], [0.5])]:
-        bb, aa = np.array(b, dtype=f32), np.array(a, dtype=f32)
-        f = R.ref_iir_new(len(bb), O._ptr(bb, O._pf), len(aa), O._ptr(aa, O._pf))
-        R.ref_iir_run(f, O._ptr(xf, O._pf), 5000, O._ptr(yr, O._pf))
-        R.ref_iir_free(f)
-        assert np.array_equal(yr, iir_oracle(b, a, xf))
+        got.append(iir_oracle(b, a, xf))
+        if R:
+            bb, aa = np.array(b, dtype=f32), np.array(a, dtype=f32)
+            f = R.ref_iir_new(len(bb), O._ptr(bb, O._pf), len(aa), O._ptr(aa, O._pf))
+            yr = np.zeros(5000, dtype=f32)
+            R.ref_iir_run(f, O._ptr(xf, O._pf), 5000, O._ptr(yr, O._pf))
+            R.ref_iir_free(f)
+            ref.append(yr)
+    _pins.expect("building_blocks", got, ref if R else None)
 
 
-@pytest.mark.skipif(not have_ref, reason="oracle/_ref not built")
 def test_decimate_audio_program_shape():
     """Int16/decimateAudio.cc: 16-tap 4:1 Decimator_int16 over 10 s of 32 kS/s audio."""
     h32000 = np.array([-0.0084477, 0.0084043, 0.0075154, 0.0064417, 0.0039647, 0.0002320, -0.0034617,
                        -0.0054143, -0.0044711, -0.0008117, 0.0038463, 0.0071423, 0.0070406, 0.0031175,
                        -0.0030506, -0.0084477], dtype=f32)
     x = (12000 * np.sin(2 * np.pi * 440 * np.arange(320000) / 32000)).astype(np.int16)
-    R = O.ref("radiodiags")
-    d = R.ref_dec16_new(16, O._ptr(h32000, O._pf), 4)
-    yr = np.zeros(80001, dtype=np.int16)
-    n = R.ref_dec16_run(d, O._ptr(x, O._pi16), len(x), O._ptr(yr, O._pi16))
-    R.ref_dec16_free(d)
-    assert n == 80000 and np.array_equal(yr[:n], dec16_oracle(h32000, 4, x))
+    got = dec16_oracle(h32000, 4, x)
+    assert got.size == 80000
+    R, ref = O.ref("radiodiags"), None
+    if R:
+        d = R.ref_dec16_new(16, O._ptr(h32000, O._pf), 4)
+        yr = np.zeros(80001, dtype=np.int16)
+        n = R.ref_dec16_run(d, O._ptr(x, O._pi16), len(x), O._ptr(yr, O._pi16))
+        R.ref_dec16_free(d)
+        ref = [yr[:n]]
+    _pins.expect("decimate_audio_program", [got], ref)

@@ -1,22 +1,23 @@
-"""The engine against the UNMODIFIED reference itself, on the GPU box: oracle/_ref holds the
-reference's own sources compiled in place (oracle/Makefile) and travels with the repository, so
-the CUDA output can be compared with IqDataProcessor -> {Am,Fm,WbFm,Ssb}Demodulator directly, not
-only with the restatement in oracle/sdr_oracle.c. All five modes, noise and modulated carriers,
-state carried over several blocks, gains, a mode switch and a reset."""
+"""The engine against the UNMODIFIED reference itself: where oracle/_ref holds the reference's own
+sources compiled in place (oracle/Makefile), the CUDA output is compared with IqDataProcessor ->
+{Am,Fm,WbFm,Ssb}Demodulator directly; elsewhere with the restatement in oracle/sdr_oracle.c and
+with the digests of the reference's output in tests/golden/reference_pins_v1.json. All five modes,
+noise and modulated carriers, state carried over several blocks, gains, a mode switch and a reset."""
 import numpy as np
 import pytest
 
 import _oracle as O
+import _pins
 import _signals as S
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(O.ref("radiodiags") is None, reason="oracle/_ref was not built")]
+pytestmark = pytest.mark.gpu
+Chain = O.RefChain if O.ref("radiodiags") is not None else O.OracleChain
 
 
 def _ref_rows(modes, iq, gains=None):
     rows = []
     for ch, m in enumerate(modes):
-        r = O.RefChain()
+        r = Chain()
         r.set_mode(int(m))
         if gains is not None and int(m):
             r.set_gain(O.MODE_TO_KIND[int(m)], float(gains[ch]))
@@ -34,9 +35,7 @@ def test_modes_match_the_compiled_reference(mode, signal):
     iq = S.noise(n, nbytes, seed=100 + mode) if signal == "noise" else S.tone_bank([mode] * n, nbytes, seed=mode)
     pcm, counts = e.demodulate(iq)
     assert (counts == 512).all()
-    exp = _ref_rows([mode] * n, iq)
-    for ch in range(n):
-        assert np.array_equal(pcm[ch], exp[ch]), "channel %d" % ch
+    _pins.expect("gpu_modes/%d/%s" % (mode, signal), list(pcm), _ref_rows([mode] * n, iq))
     e.close()
 
 
@@ -51,13 +50,14 @@ def test_long_calls_mixed_bank_gains_switch_and_reset():
     e.set_modes(modes)
     refs = []
     for ch in range(n):
-        r = O.RefChain()
+        r = Chain()
         r.set_mode(int(modes[ch]))
         r.set_gain(O.MODE_TO_KIND[int(modes[ch])], gains[ch])
         e.set_gain(ch, R.MODE_TO_KIND[int(modes[ch])], gains[ch])
         refs.append(r)
     iq = S.tone_bank(modes, 3 * blocks * 32768, seed=31)
     iq[5:] = S.noise(n - 5, iq.shape[1], seed=32)
+    got, exp = [], []
     for k in range(3):
         piece = np.ascontiguousarray(iq[:, k * blocks * 32768:(k + 1) * blocks * 32768])
         if k == 1:   # switch two channels and reset one demodulator between calls
@@ -69,6 +69,7 @@ def test_long_calls_mixed_bank_gains_switch_and_reset():
             refs[3].reset(O.MODE_TO_KIND[int(modes[3])])
         e.accept_iq_host(piece)
         pcm, _ = e.get_pcm()
-        for ch in range(n):
-            assert np.array_equal(pcm[ch], refs[ch].accept_u8(piece[ch])), "call %d channel %d" % (k, ch)
+        got.extend(pcm.copy())
+        exp.extend(refs[ch].accept_u8(piece[ch]) for ch in range(n))
+    _pins.expect("gpu_long_calls", got, exp)
     e.close()

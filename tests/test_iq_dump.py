@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 import _oracle as O
+import _pins
 import _signals as S
 
 have_ref = O.ref("radiodiags") is not None
@@ -25,22 +26,25 @@ def _drain(sock, n):
     return [sock.recv(4096) for _ in range(n)]
 
 
-@pytest.mark.skipif(not have_ref, reason="oracle/_ref not built")
 @pytest.mark.parametrize("nbytes", [32768, 4096, 5000, 2048, 1000, 8])
 def test_oracle_dump_matches_datagrams_the_reference_sends(nbytes):
+    u8 = S.noise(1, nbytes, seed=nbytes)[0]
+    u8[:16] = [0, 0, 0, 0, 0, 0, 0, 0, 255, 255, 255, 255, 255, 255, 255, 255][:min(16, nbytes)]
+    sizes = O.dump_datagrams(nbytes)
+    got = [np.array(sizes, dtype=np.int64), O.front_end(u8)]
+    if not have_ref:
+        _pins.expect("iq_dump_datagrams/%d" % nbytes, got)
+        return
     sock, port = _listener()
     try:
         r = O.RefChain(dump_port=port)
         r.set_mode(3)          # WBFM rewrites the buffer after the dump: must not show
         r.set_threshold(0)     # squelched: the dump is sent all the same
         r.set_dump(True)
-        u8 = S.noise(1, nbytes, seed=nbytes)[0]
-        u8[:16] = [0, 0, 0, 0, 0, 0, 0, 0, 255, 255, 255, 255, 255, 255, 255, 255][:min(16, nbytes)]
         r.accept_u8(u8, block=nbytes)
-        sizes = O.dump_datagrams(nbytes)
-        got = _drain(sock, len(sizes))
-        assert [len(g) for g in got] == sizes
-        assert np.array_equal(np.frombuffer(b"".join(got), dtype=np.int8), O.front_end(u8))
+        sent = _drain(sock, len(sizes))
+        _pins.expect("iq_dump_datagrams/%d" % nbytes, got,
+                     [np.array([len(g) for g in sent], dtype=np.int64), np.frombuffer(b"".join(sent), dtype=np.int8)])
         r.set_dump(False)
         r.accept_u8(u8, block=nbytes)
         sock.settimeout(0.2)

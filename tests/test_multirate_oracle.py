@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 
 import _oracle as O
+import _pins
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = np.load(os.path.join(HERE, "golden", "golden_multirate_v1.npz"))
@@ -63,9 +64,9 @@ def test_int16_unity_tap_negates():
     assert [int(v) for v in y] == exp == [-100, 200, -32767, 32767, -5]
 
 
-@pytest.mark.skipif(not have_ref, reason="oracle/_ref not built")
 @pytest.mark.parametrize("kind", [1, 2, 3, 4])
 def test_oracle_matches_compiled_reference_on_random_filters(kind):
+    got, ref = [], []
     rng = np.random.default_rng(100 + kind)
     for trial in range(12):
         factor = int(rng.integers(1, 7))
@@ -74,13 +75,12 @@ def test_oracle_matches_compiled_reference_on_random_filters(kind):
         taps = (rng.normal(0, 0.4, n_taps) * rng.choice([0.1, 1.0, 2.5])).astype(f32)
         n = int(rng.integers(1, 700))
         x = rng.integers(-32768, 32768, n).astype(np.int16 if kind >= 3 else f32)
-        a, b = O.Multirate(kind, taps, factor), O.Multirate(kind, taps, factor, impl="ref")
-        for piece in np.array_split(x, 3):
-            ya, yb = a.run(piece), b.run(piece)
-            assert ya.tobytes() == yb.tobytes(), (kind, trial)
-        a.reset()
-        b.reset()
-        assert a.run(x).tobytes() == b.run(x).tobytes()
+        for out, impl in ((got, "oracle"), (ref, "ref")) if have_ref else ((got, "oracle"),):
+            m = O.Multirate(kind, taps, factor, impl=impl)
+            out.extend(m.run(piece) for piece in np.array_split(x, 3))
+            m.reset()
+            out.append(m.run(x))
+    _pins.expect("multirate_random_filters/%d" % kind, got, ref if have_ref else None)
 
 
 REF_FILTERS = "/root/reference/radioDiags/Filters"

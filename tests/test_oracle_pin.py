@@ -2,8 +2,9 @@
 
 1. against tests/golden/golden_v1.npz -- outputs the UNMODIFIED reference produced
    when compiled in place (tests/golden/make_golden.py); always runs;
-2. against the compiled reference itself (oracle/_ref) on fresh random inputs,
-   quirk vectors, gains and ragged blocks -- runs where oracle/_ref was built;
+2. against the compiled reference itself (oracle/_ref) on seeded random inputs,
+   quirk vectors, gains and ragged blocks -- live where oracle/_ref was built, and
+   everywhere against the digests of its output in tests/golden/reference_pins_v1.json;
 3. against the md5s of the only IQ capture the reference ships
    (demodulatorResearch/yoyo.iq) -- runs where /root/reference is mounted.
 """
@@ -14,6 +15,7 @@ import numpy as np
 import pytest
 
 import _oracle as O
+import _pins
 
 GOLD = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "golden_v1.npz"))
 NAMES = {1: "am", 2: "fm", 3: "wbfm", 4: "lsb", 5: "usb"}
@@ -40,7 +42,6 @@ def test_oracle_matches_golden_research_tree(mode):
         assert np.array_equal(c.accept_s8(mode, iq[ch]), exp[ch])
 
 
-@pytest.mark.skipif(not have_ref, reason="oracle/_ref not built (needs /root/reference)")
 @pytest.mark.parametrize("mode", [1, 2, 3, 4, 5])
 @pytest.mark.parametrize("gmul", [1.0, 4.0, 1e6, 0.0])
 def test_oracle_matches_compiled_reference_noise_and_quirks(mode, gmul):
@@ -52,49 +53,54 @@ def test_oracle_matches_compiled_reference_noise_and_quirks(mode, gmul):
     u8[8193:12288:2] = 255
     kind = O.MODE_TO_KIND[mode]
     base = {1: 300.0, 2: 10185.916, 3: 40743.664, 4: 300.0}[kind]
-    r, c = O.RefChain(), O.OracleChain()
-    for x in (r, c):
+    chains = [O.OracleChain()] + ([O.RefChain()] if have_ref else [])
+    for x in chains:
         x.set_mode(mode)
         x.set_gain(kind, base * gmul)
-    assert np.array_equal(r.accept_u8(u8), c.accept_u8(u8))
+    out = [[x.accept_u8(u8)] for x in chains]
+    _pins.expect("noise_and_quirks/%d/%g" % (mode, gmul), out[0], out[1] if have_ref else None)
 
 
-@pytest.mark.skipif(not have_ref, reason="oracle/_ref not built")
 @pytest.mark.parametrize("mode", [1, 2, 3, 4])
 def test_oracle_matches_compiled_reference_ragged_blocks_and_resets(mode):
     rng = np.random.default_rng(mode)
-    r, c = O.RefChain(), O.OracleChain()
-    r.set_mode(mode)
-    c.set_mode(mode)
+    chains = [O.OracleChain()] + ([O.RefChain()] if have_ref else [])
+    out = [[] for _ in chains]
+    for x in chains:
+        x.set_mode(mode)
     kind = O.MODE_TO_KIND[mode]
     for i, n in enumerate([8, 24, 32768, 1000, 4096 + 8, 16, 2, 32768, 6]):
         u8 = rng.integers(0, 256, size=n, dtype=np.uint8)
-        assert np.array_equal(r.accept_u8(u8), c.accept_u8(u8)), "piece %d" % i
-        if i == 4:
-            r.reset(kind)
-            c.reset(kind)
+        for x, o in zip(chains, out):
+            o.append(x.accept_u8(u8))
+            if i == 4:
+                x.reset(kind)
+    _pins.expect("ragged_blocks_and_resets/%d" % mode, out[0], out[1] if have_ref else None)
 
 
-@pytest.mark.skipif(not have_ref, reason="oracle/_ref not built")
 def test_oracle_mode_switch_keeps_idle_state_like_reference():
     rng = np.random.default_rng(5)
-    r, c = O.RefChain(), O.OracleChain()
+    chains = [O.OracleChain()] + ([O.RefChain()] if have_ref else [])
+    out = [[] for _ in chains]
     for mode in [3, 2, 3, 4, 1, 5, 0, 4, 2]:
-        r.set_mode(mode)
-        c.set_mode(mode)
         u8 = rng.integers(0, 256, size=32768, dtype=np.uint8)
-        assert np.array_equal(r.accept_u8(u8), c.accept_u8(u8)), "mode %d" % mode
+        for x, o in zip(chains, out):
+            x.set_mode(mode)
+            o.append(x.accept_u8(u8))
+    _pins.expect("mode_switch", out[0], out[1] if have_ref else None)
 
 
-@pytest.mark.skipif(not have_ref, reason="oracle/_ref not built")
 @pytest.mark.parametrize("mode", [1, 2, 3, 4, 5])
 def test_oracle_matches_research_tree_direct_entry(mode):
     s8 = np.random.default_rng(70 + mode).integers(-128, 128, size=32768 * 3, dtype=np.int8)
-    d = O.RefDemod(O.MODE_TO_KIND[mode], "research")
-    if mode in (4, 5):
-        d.set_lsb(mode == 4)
+    exp = None
+    if have_ref:
+        d = O.RefDemod(O.MODE_TO_KIND[mode], "research")
+        if mode in (4, 5):
+            d.set_lsb(mode == 4)
+        exp = [d.accept(s8, block=16384)]
     c = O.OracleChain(O.VARIANT_RESEARCH)
-    assert np.array_equal(d.accept(s8, block=16384), c.accept_s8(mode, s8))
+    _pins.expect("research_direct_entry/%d" % mode, [c.accept_s8(mode, s8)], exp)
 
 
 @pytest.mark.skipif(not os.path.exists(YOYO), reason="reference tree not mounted")
@@ -120,16 +126,16 @@ def _amp_block(rng, amp, nbytes):
     return np.clip(np.round(128 + amp * rng.standard_normal(nbytes)), 0, 255).astype(np.uint8)
 
 
-@pytest.mark.skipif(not have_ref, reason="oracle/_ref not built")
 @pytest.mark.parametrize("threshold,gain", [(-200, 0), (-30, 0), (-20, 0), (-12, 3), (-6, 0), (-25, 10), (0, 0)])
 def test_squelch_oracle_matches_compiled_reference(threshold, gain):
     """Squelch::run (Squelch.cc:227-273) through IqDataProcessor: gate, one-block tail,
     tuner gain, the values handed to both signal callbacks, and the PCM that does or does
     not come out -- restatement against the reference compiled in place."""
     rng = np.random.default_rng(abs(threshold) * 7 + gain)
-    ref, orc = O.RefChain(), O.OracleChain()
+    chains = [O.OracleChain()] + ([O.RefChain()] if have_ref else [])
+    out = [[] for _ in chains]
     try:
-        for c in (ref, orc):
+        for c in chains:
             c.set_mode(2)
             c.set_threshold(threshold)
             c.set_rx_gain(gain)
@@ -137,23 +143,24 @@ def test_squelch_oracle_matches_compiled_reference(threshold, gain):
         for step, amp in enumerate([0.5, 70.0, 1.0, 0.5, 10.0, 33.0, 0.6, 0.6, 100.0, 3.0, 127.0, 0.0]):
             nbytes = 32768 if step % 3 else 4096
             blk = _amp_block(rng, amp, nbytes)
-            a = ref.accept_u8(blk, block=nbytes)
-            b = orc.accept_u8(blk)
-            assert ref.signal() == orc.signal(), "step %d" % step
-            assert np.array_equal(a, b), "step %d" % step
-            seen.add(bool(a.size))
+            for c, o in zip(chains, out):
+                o.append(c.accept_u8(blk, block=nbytes) if isinstance(c, O.RefChain) else c.accept_u8(blk))
+                o.append(np.array(c.signal(), dtype=np.int64))
+            seen.add(bool(out[0][-2].size))
         if threshold in (-30, -20, -12, -25):
             assert seen == {True, False}
+        _pins.expect("squelch/%d/%d" % (threshold, gain), out[0], out[1] if have_ref else None)
     finally:
-        ref.set_rx_gain(0)
+        if have_ref:
+            chains[1].set_rx_gain(0)
 
 
-@pytest.mark.skipif(not have_ref, reason="oracle/_ref not built")
 def test_squelch_db_table_matches_compiled_reference_over_all_magnitudes():
     """Constant-amplitude blocks sweep the detector's magnitude over its whole range, so every
     entry of DbfsCalculator's table (DbfsCalculator.cc:30-50) is exercised."""
-    ref, orc = O.RefChain(), O.OracleChain()
-    for c in (ref, orc):
+    chains = [O.OracleChain()] + ([O.RefChain()] if have_ref else [])
+    out = [[] for _ in chains]
+    for c in chains:
         c.set_mode(1)
         c.set_threshold(-18)
     for i in range(0, 128, 3):
@@ -161,9 +168,10 @@ def test_squelch_db_table_matches_compiled_reference_over_all_magnitudes():
             blk = np.empty(1024, dtype=np.uint8)
             blk[0::2] = 128 + i
             blk[1::2] = 128 - q
-            a, b = ref.accept_u8(blk, block=1024), orc.accept_u8(blk)
-            assert ref.signal() == orc.signal(), (i, q)
-            assert np.array_equal(a, b), (i, q)
+            for c, o in zip(chains, out):
+                o.append(c.accept_u8(blk, block=1024) if isinstance(c, O.RefChain) else c.accept_u8(blk))
+                o.append(np.array(c.signal(), dtype=np.int64))
+    _pins.expect("squelch_db_table", out[0], out[1] if have_ref else None)
 
 
 SQ = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "golden_squelch_v1.npz"))
