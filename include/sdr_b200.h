@@ -44,6 +44,10 @@
  *   decimate(x, &y) / interpolate(x, y[L]) per sample       sdr_filter_bank_run (blocks of samples)
  *     (Filters/Decimator.cc:281-322, Filters/Interpolator.cc interpolate)
  *   resetFilterState()                                      sdr_filter_bank_reset
+ *   new IirFilter(nb, b, na, a)                             sdr_filter_bank_create_iir
+ *     (Filters/IirFilter.cc, IirFilter.h)
+ *   IirFilter::filterData(x) per sample                     sdr_filter_bank_run (blocks of samples)
+ *   IirFilter::resetFilterState()                           sdr_filter_bank_reset
  *
  * All functions return 0 on success or a negative SDR_E_* code; none throws.
  * Calls on one engine must be serialised by the caller (the reference calls
@@ -234,16 +238,25 @@ enum {
   SDR_FILTER_DECIMATOR_F32 = 1,     /* Filters/Decimator.cc (factor 1: Filters/FirFilter.cc) */
   SDR_FILTER_INTERPOLATOR_F32 = 2,  /* Filters/Interpolator.cc; n_taps must be a multiple of factor */
   SDR_FILTER_DECIMATOR_I16 = 3,     /* Filters/Int16/Decimator_int16.cc (factor 1: FirFilter_int16.cc) */
-  SDR_FILTER_INTERPOLATOR_I16 = 4   /* Filters/Int16/Interpolator_int16.cc */
+  SDR_FILTER_INTERPOLATOR_I16 = 4,  /* Filters/Int16/Interpolator_int16.cc */
+  SDR_FILTER_IIR_F32 = 5            /* Filters/IirFilter.cc; created by sdr_filter_bank_create_iir only */
 };
 /* taps: the prototype filter h[0..n_taps-1] exactly as the reference constructor takes it. */
 int sdr_filter_bank_create(int device, int kind, uint32_t n_rows, const float *taps, uint32_t n_taps,
                            uint32_t factor, sdr_filter_bank **out);
+/* n_rows IirFilter(nb, b, na, a) objects (Direct Form I, float in and out): per sample
+ *   fir = 0; fir = fir + b[k]*x[n-k] (k = 0 .. nb-1);  r = 0; r = r + a[0]*y[n-na];
+ *   r = r + a[k]*y[n-k] (k = 1 .. na-1);  y[n] = fir - r
+ * in that order, every operation single-rounded (note a[0] meets the OLDEST output, as in the
+ * reference's ring walk). 1 <= nb <= 64, 1 <= na <= 8, 1 <= n_rows <= 65535; a run takes fewer than
+ * 2^31 samples per row and produces n_in outputs per row. NaN bit patterns may differ from x86's. */
+int sdr_filter_bank_create_iir(int device, uint32_t n_rows, const float *b, uint32_t nb, const float *a, uint32_t na,
+                               sdr_filter_bank **out);
 int sdr_filter_bank_destroy(sdr_filter_bank *b);
 int sdr_filter_bank_set_stream(sdr_filter_bank *b, void *cuda_stream);
 int sdr_filter_bank_reset(sdr_filter_bank *b);
 /* Outputs per row a run of n_in samples per row will produce now: n_in * L for an interpolator,
- * (pending + n_in) / M for a decimator (pending = samples a previous run left in the
+ * n_in for an IIR bank, (pending + n_in) / M for a decimator (pending = samples a previous run left in the
  * reference's decimationBuffer, Decimator.cc:291-303). */
 uint64_t sdr_filter_bank_out_count(const sdr_filter_bank *b, uint64_t n_in);
 /* in: [n_rows][in_stride] elements (float or int16_t by kind), n_in used per row; out:
@@ -253,7 +266,7 @@ int sdr_filter_bank_run(sdr_filter_bank *b, const void *in, uint64_t in_stride, 
                         uint64_t out_stride, uint64_t *n_out, uint32_t flags);
 int sdr_filter_bank_sync(sdr_filter_bank *b);
 /* The Q15 taps the int16 classes compute in their constructors (Decimator_int16.cc:58-62);
- * returns n_taps. */
+ * returns n_taps. SDR_E_ARG for an IIR bank (there is no Q15 IirFilter). */
 int sdr_filter_bank_taps_q15(const sdr_filter_bank *b, int16_t *q);
 uint64_t sdr_filter_bank_launch_count(const sdr_filter_bank *b);
 const char *sdr_filter_bank_last_error(const sdr_filter_bank *b);

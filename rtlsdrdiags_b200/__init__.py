@@ -33,7 +33,8 @@ ABI_SYMBOLS = ["sdr_engine_create", "sdr_engine_destroy", "sdr_set_stream", "sdr
                "sdr_bank_acquire", "sdr_bank_commit", "sdr_bank_retire", "sdr_bank_last_error",
                "sdr_filter_bank_create", "sdr_filter_bank_destroy", "sdr_filter_bank_set_stream",
                "sdr_filter_bank_reset", "sdr_filter_bank_out_count", "sdr_filter_bank_run", "sdr_filter_bank_sync",
-               "sdr_filter_bank_taps_q15", "sdr_filter_bank_launch_count", "sdr_filter_bank_last_error"]
+               "sdr_filter_bank_taps_q15", "sdr_filter_bank_launch_count", "sdr_filter_bank_last_error",
+               "sdr_filter_bank_create_iir"]
 
 
 class SdrError(RuntimeError):
@@ -124,6 +125,9 @@ def load_library(build_if_missing=True):
     L.sdr_filter_bank_launch_count.restype = u64
     L.sdr_filter_bank_last_error.argtypes = [vp]
     L.sdr_filter_bank_last_error.restype = C.c_char_p
+    L.sdr_filter_bank_create_iir.argtypes = [i32, u32, vp, u32, vp, u32, C.POINTER(vp)]
+    L.sdr_debug_filter_bank_set_iir_shape.argtypes = [vp, u32, u32]
+    L.sdr_debug_filter_bank_redo_count.argtypes = [vp, C.POINTER(u32)]
     _lib = L
     return L
 
@@ -437,6 +441,7 @@ class Bank:
 
 
 FILTER_DECIMATOR_F32, FILTER_INTERPOLATOR_F32, FILTER_DECIMATOR_I16, FILTER_INTERPOLATOR_I16 = 1, 2, 3, 4
+FILTER_IIR_F32 = 5
 
 
 class FilterBank:
@@ -507,3 +512,38 @@ class FilterBank:
 
     def sync(self):
         self._ck(self.L.sdr_filter_bank_sync(self.b))
+
+
+class IirFilterBank(FilterBank):
+    """`n_rows` independent IirFilter(len(b), b, len(a), a) objects (Filters/IirFilter.cc) on one GPU:
+    float in, float out, one output per input; 1 <= len(b) <= 64, 1 <= len(a) <= 8."""
+
+    def __init__(self, n_rows, b, a, device=0):
+        self.L = load_library()
+        self.kind, self.rows, self.factor = FILTER_IIR_F32, int(n_rows), 1
+        self.dtype = np.float32
+        hb = np.ascontiguousarray(b, dtype=np.float32)
+        ha = np.ascontiguousarray(a, dtype=np.float32)
+        self.n_taps = hb.size
+        h = C.c_void_p()
+        rc = self.L.sdr_filter_bank_create_iir(int(device), self.rows, hb.ctypes.data_as(C.c_void_p), hb.size,
+                                               ha.ctypes.data_as(C.c_void_p), ha.size, C.byref(h))
+        if rc != 0:
+            raise SdrError("sdr_filter_bank_create_iir failed (%d): %s" % (rc, self.L.sdr_filter_bank_last_error(None).decode()))
+        self.b = h
+
+    def taps_q15(self):
+        raise SdrError("there is no Q15 IirFilter")
+
+    # ---- diagnostics (tests, tuning) ----
+    def debug_set_iir_shape(self, seg_count=0, warm=None):
+        """Segmentation: seg_count 0 = chosen per call, else a power of two <= 32 segments per row;
+        warm = samples a segment warms up on (rounded up to blocks of 32), None = the bank's own."""
+        self._ck(self.L.sdr_debug_filter_bank_set_iir_shape(self.b, int(seg_count),
+                                                            0xFFFFFFFF if warm is None else int(warm)))
+
+    def debug_redo_count(self):
+        """Segments redone serially since the bank was created. Synchronises."""
+        n = C.c_uint32()
+        self._ck(self.L.sdr_debug_filter_bank_redo_count(self.b, C.byref(n)))
+        return n.value

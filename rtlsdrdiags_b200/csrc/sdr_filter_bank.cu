@@ -12,6 +12,7 @@
 
 #include "../../include/sdr_b200.h"
 #include "sdr_filter_bank.cuh"
+#include "sdr_iir_bank.cuh"
 
 using namespace sdr;
 
@@ -31,6 +32,12 @@ struct sdr_filter_bank {
   uint64_t cap_in = 0, cap_out = 0;
   uint64_t launches = 0;
   std::string err;
+  // SDR_FILTER_IIR_F32: taps, the warm-up the taps need (~0u: the response does not decay, so no
+  // segmentation), the diagnostic overrides (seg 0 / warm ~0u = automatic) and the redo counter
+  std::vector<float> iir_b, iir_a;
+  uint32_t iir_warm = 0, dbg_seg = 0, dbg_warm = ~0u;
+  uint64_t resident_lanes = 0;
+  uint32_t *d_redo = nullptr;
 };
 
 namespace {
@@ -103,6 +110,88 @@ static size_t fb_plan(const sdr_filter_bank *b, FilterBankParams &p, uint32_t &t
   return smem;
 }
 
+// Warm-up of the IIR bank's segments: the zero-input recurrence in double, from each unit initial
+// state, with IirFilter's tap order; W = the first step after which every response stays below
+// 2^-64 (for a = {-0.95}: 865). Two states that differ by at most their own size then agree far
+// below float resolution. A response that has not decayed within IIR_WARM_CAP steps (marginal or
+// unstable filters, or very slow poles) returns ~0u: such banks run one segment per row.
+static constexpr int IIR_WARM_CAP = 8192;
+static uint32_t iir_warm_up(const float *a, uint32_t na) {
+  const double tiny = ldexp(1.0, -64);
+  int last = 0;  // last step (1-based) whose response was not below 2^-64
+  for (uint32_t i = 0; i < na; ++i) {
+    double h[IIR_MAX_NA] = {};  // h[0] = y[n-1]
+    h[i] = 1.0;
+    for (int n = 1; n <= 2 * IIR_WARM_CAP; ++n) {
+      double r = 0.0 + (double)a[0] * h[na - 1];
+      for (uint32_t k = 1; k < na; ++k) r = r + (double)a[k] * h[k - 1];
+      const double y = 0.0 - r;
+      for (uint32_t k = na - 1; k > 0; --k) h[k] = h[k - 1];
+      h[0] = y;
+      if (!(fabs(y) < tiny)) last = n;
+    }
+  }
+  return last + 1 > IIR_WARM_CAP ? ~0u : (uint32_t)(last + 1);
+}
+
+typedef void (*IirKernel)(IirBankParams);
+template <int NB>
+static IirKernel iir_kernel_nb(uint32_t na) {
+  switch (na) {
+    case 1: return iir_bank_kernel<1, NB>;
+    case 2: return iir_bank_kernel<2, NB>;
+    case 3: return iir_bank_kernel<3, NB>;
+    case 4: return iir_bank_kernel<4, NB>;
+    case 5: return iir_bank_kernel<5, NB>;
+    case 6: return iir_bank_kernel<6, NB>;
+    case 7: return iir_bank_kernel<7, NB>;
+    default: return iir_bank_kernel<8, NB>;
+  }
+}
+static IirKernel iir_kernel(uint32_t nb, uint32_t na) {
+  return nb == 1 ? iir_kernel_nb<1>(na) : nb == 2 ? iir_kernel_nb<2>(na) : iir_kernel_nb<0>(na);
+}
+
+// One IIR call: S segments per row (a power of two <= 32) so that rows x S lanes fill the GPU
+// without a second wave, each at least four warm-ups long; no empty segments in the middle.
+static int iir_run(sdr_filter_bank *b, const float *d_in, uint64_t istr, float *d_out, uint64_t ostr, uint32_t n) {
+  const uint32_t blocks = (n + IIR_BLK - 1) / IIR_BLK;
+  const uint32_t warm = b->dbg_warm != ~0u ? b->dbg_warm : b->iir_warm;
+  const uint32_t warm_r = warm == ~0u ? ~0u : (warm + IIR_BLK - 1) / IIR_BLK * IIR_BLK;
+  uint32_t S = 1;
+  if (b->dbg_seg) {
+    S = b->dbg_seg;
+  } else if (warm_r != ~0u) {
+    const uint32_t min_blocks = 4 * (warm_r / IIR_BLK > 0 ? warm_r / IIR_BLK : 1);
+    while (S < 32 && (uint64_t)b->rows * 2 * S <= b->resident_lanes && blocks / (2 * S) >= min_blocks) S *= 2;
+  }
+  while (S > 1 && (blocks + S - 1) / S * (S - 1) >= blocks) S /= 2;
+  IirBankParams p;
+  p.in = d_in;
+  p.out = d_out;
+  p.carry_in = (const float *)b->d_carry[b->cur];
+  p.carry_out = (float *)b->d_carry[b->cur ^ 1];
+  p.redo = b->d_redo;
+  p.in_stride = istr;
+  p.out_stride = ostr;
+  p.n = n;
+  p.rows = b->rows;
+  p.nb = (uint32_t)b->iir_b.size();
+  p.na = (uint32_t)b->iir_a.size();
+  p.C = b->C;
+  p.seg_log2 = 0;
+  while ((1u << p.seg_log2) < S) ++p.seg_log2;
+  p.seg_len = (blocks + S - 1) / S * IIR_BLK;
+  p.warm = S == 1 ? 0u : (warm_r == ~0u ? p.seg_len * S : warm_r);  // ~0u with a forced S: start at the head
+  memset(p.b, 0, sizeof p.b);
+  memset(p.a, 0, sizeof p.a);
+  memcpy(p.b, b->iir_b.data(), 4 * (size_t)p.nb);
+  memcpy(p.a, b->iir_a.data(), 4 * (size_t)p.na);
+  const uint64_t lanes = (uint64_t)b->rows << p.seg_log2;
+  iir_kernel(p.nb, p.na)<<<(unsigned)((lanes + 31) / 32), IIR_THREADS, 0, b->stream>>>(p);
+  return SDR_OK;
+}
+
 extern "C" {
 
 int sdr_filter_bank_create(int device, int kind, uint32_t n_rows, const float *taps, uint32_t n_taps,
@@ -173,6 +262,48 @@ int sdr_filter_bank_create(int device, int kind, uint32_t n_rows, const float *t
   return SDR_OK;
 }
 
+/* IirFilter(nb, b, na, a) (Filters/IirFilter.cc) for every row */
+int sdr_filter_bank_create_iir(int device, uint32_t n_rows, const float *b_taps, uint32_t nb, const float *a_taps,
+                               uint32_t na, sdr_filter_bank **out) {
+  if (!out) return fb_fail(nullptr, SDR_E_ARG, "out is NULL");
+  *out = nullptr;
+  if (!b_taps || !a_taps || nb < 1 || nb > IIR_MAX_NB || na < 1 || na > IIR_MAX_NA || n_rows == 0 || n_rows > 65535)
+    return fb_fail(nullptr, SDR_E_ARG, "IIR bank: taps must be set, 1 <= nb <= 64, 1 <= na <= 8, 1 <= n_rows <= 65535");
+  int count = 0;
+  if (cudaGetDeviceCount(&count) != cudaSuccess || device < 0 || device >= count)
+    return fb_fail(nullptr, SDR_E_CUDA, "no usable CUDA device (there is no CPU fallback)");
+  FB_CK(nullptr, cudaSetDevice(device));
+  sdr_filter_bank *b = new sdr_filter_bank;
+  b->device = device;
+  b->kind = SDR_FILTER_IIR_F32;
+  b->rows = n_rows;
+  b->N = nb;
+  b->F = 1;
+  b->esize = 4;
+  b->C = (nb - 1) + na;  // per row: the last nb - 1 inputs, then the last na outputs
+  b->iir_b.assign(b_taps, b_taps + nb);
+  b->iir_a.assign(a_taps, a_taps + na);
+  b->iir_warm = iir_warm_up(a_taps, na);
+  if (b->iir_warm != ~0u && b->iir_warm < na) b->iir_warm = na;  // the compared state must be made of computed outputs
+  int per_sm = 0, sms = 0;
+  cudaError_t ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, iir_kernel(nb, na), IIR_THREADS, 0);
+  if (ce == cudaSuccess) ce = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+  if (ce != cudaSuccess) { delete b; return fb_fail(nullptr, SDR_E_CUDA, "IIR bank: occupancy query", ce); }
+  b->resident_lanes = (uint64_t)(per_sm > 0 ? per_sm : 1) * (uint64_t)sms * 32;
+  ce = cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking);
+  if (ce != cudaSuccess) { delete b; return fb_fail(nullptr, SDR_E_CUDA, "cudaStreamCreate", ce); }
+  b->stream = b->own_stream;
+  const size_t cbytes = (size_t)b->C * n_rows * 4;
+  if ((ce = cudaMalloc(&b->d_carry[0], cbytes)) != cudaSuccess || (ce = cudaMalloc(&b->d_carry[1], cbytes)) != cudaSuccess ||
+      (ce = cudaMalloc(&b->d_redo, 4)) != cudaSuccess || (ce = cudaMemset(b->d_carry[0], 0, cbytes)) != cudaSuccess ||
+      (ce = cudaMemset(b->d_carry[1], 0, cbytes)) != cudaSuccess || (ce = cudaMemset(b->d_redo, 0, 4)) != cudaSuccess) {
+    sdr_filter_bank_destroy(b);
+    return fb_fail(nullptr, ce == cudaErrorMemoryAllocation ? SDR_E_NOMEM : SDR_E_CUDA, "filter bank allocation", ce);
+  }
+  *out = b;
+  return SDR_OK;
+}
+
 int sdr_filter_bank_destroy(sdr_filter_bank *b) {
   if (!b) return SDR_E_ARG;
   cudaSetDevice(b->device);
@@ -182,6 +313,7 @@ int sdr_filter_bank_destroy(sdr_filter_bank *b) {
   cudaFree(b->d_carry[1]);
   cudaFree(b->d_in);
   cudaFree(b->d_out);
+  cudaFree(b->d_redo);
   if (b->own_stream) cudaStreamDestroy(b->own_stream);
   delete b;
   return SDR_OK;
@@ -211,7 +343,7 @@ uint64_t sdr_filter_bank_out_count(const sdr_filter_bank *b, uint64_t n_in) {
 }
 
 int sdr_filter_bank_taps_q15(const sdr_filter_bank *b, int16_t *q) {
-  if (!b || !q) return SDR_E_ARG;
+  if (!b || !q || b->kind == SDR_FILTER_IIR_F32) return SDR_E_ARG;  // there is no Q15 IirFilter
   memcpy(q, b->q15.data(), 2 * (size_t)b->N);
   return (int)b->N;
 }
@@ -224,6 +356,7 @@ int sdr_filter_bank_run(sdr_filter_bank *b, const void *in, uint64_t in_stride, 
   if (n_in == 0) return SDR_OK;
   if (!in || (n_out && !out) || in_stride < n_in || out_stride < n_out) return fb_fail(b, SDR_E_ARG, "bad buffer, stride or count");
   if (n_in > (1ull << 40)) return fb_fail(b, SDR_E_TOO_LONG, "n_in too large");
+  if (b->kind == SDR_FILTER_IIR_F32 && n_in >= (1ull << 31)) return fb_fail(b, SDR_E_TOO_LONG, "IIR bank: n_in must be below 2^31");
   FB_CK(b, cudaSetDevice(b->device));
   const bool host = !(flags & SDR_IQ_DEVICE);
   const void *d_in = in;
@@ -255,6 +388,9 @@ int sdr_filter_bank_run(sdr_filter_bank *b, const void *in, uint64_t in_stride, 
     ostr = n_out;
   }
 
+  if (b->kind == SDR_FILTER_IIR_F32) {
+    iir_run(b, (const float *)d_in, istr, (float *)d_out, ostr, (uint32_t)n_in);
+  } else {
   FilterBankParams p;
   p.in = d_in;
   p.out = d_out;
@@ -302,6 +438,7 @@ int sdr_filter_bank_run(sdr_filter_bank *b, const void *in, uint64_t in_stride, 
 #undef FB_LAUNCH_INT
 #undef FB_LAUNCH_DEC
 #undef FB_LAUNCH
+  }
   FB_CK(b, cudaGetLastError());
   ++b->launches;
   b->cur ^= 1;
@@ -326,6 +463,25 @@ uint64_t sdr_filter_bank_launch_count(const sdr_filter_bank *b) { return b ? b->
 
 const char *sdr_filter_bank_last_error(const sdr_filter_bank *b) {
   return b ? b->err.c_str() : g_fb_create_error.c_str();
+}
+
+// Diagnostics (not part of include/sdr_b200.h): the IIR bank's segmentation -- seg_count 0 = chosen
+// per call, else a power of two <= 32; warm = samples a segment s > 0 warms up on (rounded up to
+// blocks of 32; ~0u = the bank's own) -- and how many segments were redone serially so far
+// (synchronises). Tests shrink the warm-up to force the redo path.
+int sdr_debug_filter_bank_set_iir_shape(sdr_filter_bank *b, uint32_t seg_count, uint32_t warm) {
+  if (!b || b->kind != SDR_FILTER_IIR_F32 || seg_count > 32 || (seg_count & (seg_count - 1))) return SDR_E_ARG;
+  b->dbg_seg = seg_count;
+  b->dbg_warm = warm;
+  return SDR_OK;
+}
+
+int sdr_debug_filter_bank_redo_count(sdr_filter_bank *b, uint32_t *count) {
+  if (!b || !count || b->kind != SDR_FILTER_IIR_F32) return SDR_E_ARG;
+  FB_CK(b, cudaSetDevice(b->device));
+  FB_CK(b, cudaMemcpyAsync(count, b->d_redo, 4, cudaMemcpyDeviceToHost, b->stream));
+  FB_CK(b, cudaStreamSynchronize(b->stream));
+  return SDR_OK;
 }
 
 }  // extern "C"
