@@ -27,17 +27,20 @@
  *     (src_diags/IqDataProcessor.cc:284-295)
  *   radio_adjustableReceiveGainInDb (IqDataProcessor.cc:8) sdr_set_receive_gain_db
  *   signal-state / signal-magnitude callbacks              sdr_enable_signal_reports,
- *     (src_diags/IqDataProcessor.cc:771-790)                sdr_get_signal
- *   IqDataProcessor::enableIqDump / disableIqDump          sdr_set_iq_dump
+ *     (src_diags/IqDataProcessor.cc:771-790)                sdr_get_signal (direct calls),
+ *                                                           sdr_ingest_retired_signal (ring),
+ *                                                           sdr_bank_retired_signal (bank)
+ *   IqDataProcessor::enableIqDump / disableIqDump          sdr_set_iq_dump, sdr_bank_set_iq_dump
  *     (src_diags/IqDataProcessor.cc:633-669)
- *   networkInterfacePtr->sendData(signedBufferPtr, n)      sdr_get_iq_dump / sdr_iq_dump_device
- *     (IqDataProcessor.cc:756-760, UdpClient.cc:173-241)
+ *   networkInterfacePtr->sendData(signedBufferPtr, n)      sdr_get_iq_dump / sdr_iq_dump_device,
+ *     (IqDataProcessor.cc:756-760, UdpClient.cc:173-241)    sdr_ingest_retired_iq_dump,
+ *                                                           sdr_bank_retired_iq_dump
  *   DataConsumer::acceptData(ts, buf, n) + consumer thread  sdr_ingest_accept / _acquire+_commit,
  *     (src_diags/DataConsumer.cc:220-261, 318-352)           sdr_ingest_retire, sdr_ingest_stats
  *   Radio's demodulator objects, one set per radio, and    sdr_bank_create, sdr_bank_set_mode(s),
  *     one DataConsumer feeding them (Radio.cc:150-187,       sdr_bank_acquire + sdr_bank_commit,
- *     DataConsumer.cc:220-352) -- for radios spread over     sdr_bank_retire
- *     several GPUs of one box
+ *     DataConsumer.cc:220-352) -- for radios spread over     sdr_bank_retire, sdr_bank_set_receive_gain_db,
+ *     several GPUs of one box                                sdr_bank_enable_signal_reports
  *   new Decimator / Interpolator / Decimator_int16 /        sdr_filter_bank_create
  *     Interpolator_int16 (N, taps, factor)
  *     (Filters/Decimator.cc:41-76, Filters/Interpolator.cc:39-61, Filters/Int16/*.cc)
@@ -122,7 +125,9 @@ int sdr_set_receive_gain_db(sdr_engine *e, uint32_t channel, uint32_t gain_db);
  * close (what enableSignalNotification / enableSignalMagnitudeNotification ask for). */
 int sdr_enable_signal_reports(sdr_engine *e, int on);
 /* Gate and mean magnitude of the last call, [n_channels] each; either may be NULL.
- * Synchronises. Fails with SDR_E_ARG if the last call did not run the squelch. */
+ * Synchronises. Fails with SDR_E_ARG if the last call did not run the squelch. With an ingest
+ * ring in use this is the newest committed tick, not the retired one: see
+ * sdr_ingest_retired_signal. */
 int sdr_get_signal(sdr_engine *e, uint8_t *allowed, uint32_t *magnitude);
 
 /* IQ dump (IqDataProcessor.cc:756-760): keep, for the channels it is enabled on, the block
@@ -135,7 +140,9 @@ int sdr_set_iq_dump(sdr_engine *e, uint32_t channel, int on);
  * NULL to ask for the size only. Synchronises. SDR_E_ARG if the channel was not dumped. */
 int sdr_get_iq_dump(sdr_engine *e, uint32_t channel, int8_t *out, uint64_t capacity, uint64_t *n_bytes);
 /* Device-resident dump of the last call: n_rows rows, row_stride apart, in ascending channel
- * order of the enabled channels. */
+ * order of the enabled channels. The engine rotates between three dump buffers, so ask again
+ * after every sdr_accept_iq. With an ingest ring in use, both describe the newest committed tick:
+ * see sdr_ingest_retired_iq_dump. */
 int sdr_iq_dump_device(sdr_engine *e, int8_t **rows, uint64_t *row_stride, uint32_t *n_rows);
 
 /* One block for every channel: iq is [n_channels][channel_stride] bytes of
@@ -187,6 +194,18 @@ int sdr_ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes_per_chan
  * next sdr_ingest_acquire / sdr_ingest_accept. SDR_E_EMPTY if nothing is in flight. */
 int sdr_ingest_retire(sdr_ingest *q, uint32_t *timestamp, const int16_t **pcm, uint32_t *samples_per_row,
                       const uint32_t **counts);
+/* The signal reports and IQ dump of each tick (IqDataProcessor.cc:756-760, 771-790), as the
+ * squelch and dump settings stood at its commit (setters called between commits take effect at the
+ * next one). Both are about the tick the last sdr_ingest_retire returned, and their pointers (pinned
+ * host memory) stay valid until that slot is acquired again. SDR_E_EMPTY if nothing was retired yet
+ * or that slot was committed again since. */
+/* Gate and mean magnitude of the last retired tick, [n_channels] each; either may be NULL.
+ * SDR_E_ARG if that tick ran no squelch (no threshold that can close and reports off at its commit). */
+int sdr_ingest_retired_signal(const sdr_ingest *q, const uint8_t **allowed, const uint32_t **magnitude);
+/* IQ dump of the last retired tick: n_rows rows of *n_bytes (that tick's bytes_per_channel) signed, rotated
+ * bytes, *row_stride apart, for channels[0..n_rows) in ascending order; n_rows = 0 if none was dumped. */
+int sdr_ingest_retired_iq_dump(const sdr_ingest *q, const int8_t **rows, uint64_t *row_stride, uint64_t *n_bytes,
+                               const uint32_t **channels, uint32_t *n_rows);
 /* lastTimeStamp and shortBlockCount (DataConsumer.cc:282-283), ticks committed, ticks in flight */
 int sdr_ingest_stats(const sdr_ingest *q, uint32_t *last_timestamp, uint32_t *short_block_count, uint64_t *ticks,
                      uint32_t *in_flight);
@@ -214,6 +233,10 @@ int sdr_bank_set_modes(sdr_bank *b, const uint8_t *modes /* [n_channels] */);
 int sdr_bank_set_gain(sdr_bank *b, uint32_t channel, int kind, float gain);
 int sdr_bank_reset(sdr_bank *b, uint32_t channel, int kind);
 int sdr_bank_set_squelch_threshold(sdr_bank *b, uint32_t channel, int32_t threshold_dbfs);
+int sdr_bank_set_receive_gain_db(sdr_bank *b, uint32_t channel, uint32_t gain_db);
+int sdr_bank_set_iq_dump(sdr_bank *b, uint32_t channel, int on);
+/* sdr_enable_signal_reports on every shard */
+int sdr_bank_enable_signal_reports(sdr_bank *b, int on);
 /* The next free tick array, [n_channels][*channel_stride] bytes of pinned host memory. */
 int sdr_bank_acquire(sdr_bank *b, void **iq, uint64_t *channel_stride);
 /* Queue the acquired tick on every device (flags: SDR_IQ_U8_OFFSET or SDR_IQ_S8_ROTATED). A tick
@@ -223,6 +246,14 @@ int sdr_bank_commit(sdr_bank *b, uint32_t timestamp, uint64_t bytes_per_channel,
  * (pinned host memory, valid until the slot is acquired again) and counts[n_channels]. */
 int sdr_bank_retire(sdr_bank *b, uint32_t *timestamp, const int16_t **pcm, uint32_t *samples_per_row,
                     const uint32_t **counts);
+/* The signal reports and IQ dump of the tick the last sdr_bank_retire returned, gathered like its PCM
+ * into pinned arrays of the slot (valid until the slot is acquired again); the rules and codes are
+ * those of sdr_ingest_retired_signal / sdr_ingest_retired_iq_dump. The gate and magnitudes are
+ * [n_channels]; SDR_E_ARG unless every shard ran the squelch for that tick. The dump rows are in
+ * ascending global channel order across shards. */
+int sdr_bank_retired_signal(sdr_bank *b, const uint8_t **allowed, const uint32_t **magnitude);
+int sdr_bank_retired_iq_dump(sdr_bank *b, const int8_t **rows, uint64_t *row_stride, uint64_t *n_bytes,
+                             const uint32_t **channels, uint32_t *n_rows);
 /* Text of the last error on this bank (or of the last failed create if b is NULL). */
 const char *sdr_bank_last_error(const sdr_bank *b);
 
@@ -261,7 +292,8 @@ int sdr_filter_bank_reset(sdr_filter_bank *b);
 uint64_t sdr_filter_bank_out_count(const sdr_filter_bank *b, uint64_t n_in);
 /* in: [n_rows][in_stride] elements (float or int16_t by kind), n_in used per row; out:
  * [n_rows][out_stride]. flags: SDR_IQ_HOST (copied in and out, returns when out is filled) or
- * SDR_IQ_DEVICE (queued on the bank's stream). *n_out = outputs written per row. */
+ * SDR_IQ_DEVICE (queued on the bank's stream; the bank's own stream is a blocking one, so it runs
+ * after what was queued before on the legacy default stream). *n_out = outputs written per row. */
 int sdr_filter_bank_run(sdr_filter_bank *b, const void *in, uint64_t in_stride, uint64_t n_in, void *out,
                         uint64_t out_stride, uint64_t *n_out, uint32_t flags);
 int sdr_filter_bank_sync(sdr_filter_bank *b);

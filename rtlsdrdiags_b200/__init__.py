@@ -34,7 +34,9 @@ ABI_SYMBOLS = ["sdr_engine_create", "sdr_engine_destroy", "sdr_set_stream", "sdr
                "sdr_filter_bank_create", "sdr_filter_bank_destroy", "sdr_filter_bank_set_stream",
                "sdr_filter_bank_reset", "sdr_filter_bank_out_count", "sdr_filter_bank_run", "sdr_filter_bank_sync",
                "sdr_filter_bank_taps_q15", "sdr_filter_bank_launch_count", "sdr_filter_bank_last_error",
-               "sdr_filter_bank_create_iir"]
+               "sdr_filter_bank_create_iir", "sdr_ingest_retired_signal", "sdr_ingest_retired_iq_dump",
+               "sdr_bank_set_receive_gain_db", "sdr_bank_set_iq_dump", "sdr_bank_enable_signal_reports",
+               "sdr_bank_retired_signal", "sdr_bank_retired_iq_dump"]
 
 
 class SdrError(RuntimeError):
@@ -84,6 +86,9 @@ def load_library(build_if_missing=True):
     L.sdr_ingest_commit.argtypes = [vp, u32, u64, u32]
     L.sdr_ingest_retire.argtypes = [vp, C.POINTER(u32), C.POINTER(vp), C.POINTER(u32), C.POINTER(vp)]
     L.sdr_ingest_stats.argtypes = [vp, C.POINTER(u32), C.POINTER(u32), C.POINTER(u64), C.POINTER(u32)]
+    L.sdr_ingest_retired_signal.argtypes = [vp, C.POINTER(vp), C.POINTER(vp)]
+    L.sdr_ingest_retired_iq_dump.argtypes = [vp, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64), C.POINTER(vp),
+                                             C.POINTER(u32)]
     L.sdr_set_launch_shape.argtypes = [vp, i32, u32, u32]
     L.sdr_launch_count.argtypes = [vp]
     L.sdr_launch_count.restype = u64
@@ -107,6 +112,12 @@ def load_library(build_if_missing=True):
     L.sdr_bank_set_gain.argtypes = [vp, u32, i32, C.c_float]
     L.sdr_bank_reset.argtypes = [vp, u32, i32]
     L.sdr_bank_set_squelch_threshold.argtypes = [vp, u32, C.c_int32]
+    L.sdr_bank_set_receive_gain_db.argtypes = [vp, u32, u32]
+    L.sdr_bank_set_iq_dump.argtypes = [vp, u32, i32]
+    L.sdr_bank_enable_signal_reports.argtypes = [vp, i32]
+    L.sdr_bank_retired_signal.argtypes = [vp, C.POINTER(vp), C.POINTER(vp)]
+    L.sdr_bank_retired_iq_dump.argtypes = [vp, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64), C.POINTER(vp),
+                                           C.POINTER(u32)]
     L.sdr_bank_acquire.argtypes = [vp, C.POINTER(vp), C.POINTER(u64)]
     L.sdr_bank_commit.argtypes = [vp, u32, u64, u32]
     L.sdr_bank_retire.argtypes = [vp, C.POINTER(u32), C.POINTER(vp), C.POINTER(u32), C.POINTER(vp)]
@@ -130,6 +141,27 @@ def load_library(build_if_missing=True):
     L.sdr_debug_filter_bank_redo_count.argtypes = [vp, C.POINTER(u32)]
     _lib = L
     return L
+
+
+def _retired_signal(fn, handle, n, ck):
+    """(allowed [n] bool, magnitude [n] uint32) through sdr_ingest_retired_signal / sdr_bank_retired_signal."""
+    a, m = C.c_void_p(), C.c_void_p()
+    ck(fn(handle, C.byref(a), C.byref(m)))
+    allowed = np.frombuffer((C.c_uint8 * n).from_address(a.value), dtype=np.uint8).astype(bool)
+    mag = np.frombuffer((C.c_uint32 * n).from_address(m.value), dtype=np.uint32).copy()
+    return allowed, mag
+
+
+def _retired_iq_dump(fn, handle, ck):
+    """{channel: int8 row} through sdr_ingest_retired_iq_dump / sdr_bank_retired_iq_dump (copies)."""
+    rows, stride, nb, chans, nr = C.c_void_p(), C.c_uint64(), C.c_uint64(), C.c_void_p(), C.c_uint32()
+    ck(fn(handle, C.byref(rows), C.byref(stride), C.byref(nb), C.byref(chans), C.byref(nr)))
+    if nr.value == 0:
+        return {}
+    ch = np.frombuffer((C.c_uint32 * nr.value).from_address(chans.value), dtype=np.uint32)
+    buf = np.frombuffer((C.c_int8 * (nr.value * stride.value)).from_address(rows.value), dtype=np.int8)
+    buf = buf.reshape(nr.value, stride.value)
+    return {int(c): buf[i, :nb.value].copy() for i, c in enumerate(ch)}
 
 
 class Engine:
@@ -360,6 +392,15 @@ class Ingest:
         pcm = pcm.reshape(n, samples.value)
         return ts.value, (pcm.copy() if copy else pcm), (counts.copy() if copy else counts)
 
+    def retired_signal(self):
+        """(allowed [n] bool, magnitude [n] uint32) of the last retired tick: the signal-state and
+        signal-magnitude reports (IqDataProcessor.cc:771-790). Raises if that tick ran no squelch."""
+        return _retired_signal(self.L.sdr_ingest_retired_signal, self.q, self.e.n, self.e._ck)
+
+    def retired_iq_dump(self):
+        """{channel: int8 array} of the last retired tick's IQ dump (IqDataProcessor.cc:756-760)."""
+        return _retired_iq_dump(self.L.sdr_ingest_retired_iq_dump, self.q, self.e._ck)
+
     def stats(self):
         ts, short, ticks, fl = C.c_uint32(), C.c_uint32(), C.c_uint64(), C.c_uint32()
         self.e._ck(self.L.sdr_ingest_stats(self.q, C.byref(ts), C.byref(short), C.byref(ticks), C.byref(fl)))
@@ -418,6 +459,24 @@ class Bank:
 
     def set_squelch_threshold(self, channel, dbfs):
         self._ck(self.L.sdr_bank_set_squelch_threshold(self.b, channel, int(dbfs)))
+
+    def set_receive_gain_db(self, channel, gain_db):
+        self._ck(self.L.sdr_bank_set_receive_gain_db(self.b, channel, int(gain_db)))
+
+    def enable_signal_reports(self, on=True):
+        self._ck(self.L.sdr_bank_enable_signal_reports(self.b, int(bool(on))))
+
+    def set_iq_dump(self, channel, on=True):
+        self._ck(self.L.sdr_bank_set_iq_dump(self.b, channel, int(bool(on))))
+
+    def retired_signal(self):
+        """(allowed [n] bool, magnitude [n] uint32) of the last retired tick, gathered over all shards.
+        Raises unless every shard ran the squelch for that tick."""
+        return _retired_signal(self.L.sdr_bank_retired_signal, self.b, self.n, self._ck)
+
+    def retired_iq_dump(self):
+        """{global channel: int8 array} of the last retired tick's IQ dump."""
+        return _retired_iq_dump(self.L.sdr_bank_retired_iq_dump, self.b, self._ck)
 
     def acquire(self):
         """The next free tick as a writable [n_channels][block_bytes] uint8 view of pinned memory."""

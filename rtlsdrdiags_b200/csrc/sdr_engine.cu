@@ -111,7 +111,9 @@ struct sdr_engine {
   std::vector<uint32_t> rx_gain_db; // radio_adjustableReceiveGainInDb per radio
   bool squelch_dirty = false, squelch_armed = false, signal_reports = false;
   int32_t *d_threshold = nullptr;
-  uint32_t *d_rx_gain = nullptr, *d_magnitude = nullptr;
+  uint32_t *d_rx_gain = nullptr;
+  uint32_t *d_magnitude = nullptr;  // [RING_MAX][n], entry call % RING_MAX, like d_allowed
+  uint32_t *magnitude_of(uint64_t call) const { return d_magnitude + (size_t)(call % RING_MAX) * n; }
   uint8_t *d_tracking = nullptr, *d_allowed[RING_MAX] = {};
   int32_t *d_db_table = nullptr;
   bool last_gated = false;  // the last accept ran the squelch kernel with the gate in force
@@ -123,10 +125,14 @@ struct sdr_engine {
   std::vector<uint8_t> dump_on;
   std::vector<uint32_t> dump_list;
   bool dump_dirty = false;
+  uint32_t dump_count = 0;    // channels with dump_on set: the rows the next call dumps
   uint32_t *d_dump_list = nullptr;
-  int8_t *d_dump = nullptr;
-  size_t dump_rows = 0;       // rows d_dump holds
+  int8_t *d_dump = nullptr;   // [RING_MAX][dump_rows][max_bytes], entry call % RING_MAX
+  size_t dump_rows = 0;       // rows each entry of d_dump holds
   uint64_t dump_bytes = 0;    // bytes per channel of the last dump (0 = none)
+  int8_t *dump_of(uint64_t call) const { return d_dump + (size_t)(call % RING_MAX) * dump_rows * max_bytes; }
+  // the ingest ring's device->host stream, which copies out of d_dump: drained before d_dump is freed
+  cudaStream_t dump_reader = nullptr;
 
   // SDR_TRACE=1: per call [FIR start, FIR end, dc_block start, dc_block end] in globaltimer ns (tools/probe_timeline.py)
   unsigned long long *d_trace = nullptr;
@@ -944,12 +950,13 @@ int run_iq_dump(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint64_t b
       if (e->dump_on[ch]) e->dump_list.push_back(ch);
     if (e->dump_list.size() > e->dump_rows) {
       SDR_CK(e, cudaStreamSynchronize(e->stream));
+      if (e->dump_reader) SDR_CK(e, cudaStreamSynchronize(e->dump_reader));
       cudaFree(e->d_dump);
       cudaFree(e->d_dump_list);
       e->d_dump = nullptr;
       e->d_dump_list = nullptr;
       e->dump_rows = e->dump_list.size();
-      SDR_CK(e, cudaMalloc(&e->d_dump, e->dump_rows * e->max_bytes));
+      SDR_CK(e, cudaMalloc(&e->d_dump, sdr_engine::RING_MAX * e->dump_rows * e->max_bytes));
       SDR_CK(e, cudaMalloc(&e->d_dump_list, e->dump_rows * 4));
     }
     if (!e->dump_list.empty()) {
@@ -967,7 +974,13 @@ int run_iq_dump(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint64_t b
   d.fmt = fmt;
   d.list = e->d_dump_list;
   d.n_list = (uint32_t)e->dump_list.size();
-  d.out = e->d_dump;
+  // Ring entry seq % RING_MAX (so are the squelch's gate and magnitude, see run_squelch). A direct
+  // caller reads entry seq - 1 on `stream`, in order. The ingest ring reads tick k's entry on its
+  // d2h stream, after tick k's ev_comp and before its ev_done, and ingest_commit makes tick k+2's
+  // work on `stream` wait for tick k's ev_done. Tick k+3, the next to write this entry, is queued on
+  // `stream` after tick k+2, so its kernels start only once tick k's copies are over: three
+  // entries are enough however deep the ingest ring is.
+  d.out = e->dump_of(e->seq);
   d.out_stride = e->max_bytes;
   const uint64_t pieces = bytes / 16;
   uint32_t gx = (uint32_t)std::min<uint64_t>((pieces + 255) / 256, 64);
@@ -990,14 +1003,14 @@ int run_squelch(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint64_t b
     if ((armed || e->signal_reports) && !e->d_tracking) {
       SDR_CK(e, cudaMalloc(&e->d_threshold, (size_t)e->n * 4));
       SDR_CK(e, cudaMalloc(&e->d_rx_gain, (size_t)e->n * 4));
-      SDR_CK(e, cudaMalloc(&e->d_magnitude, (size_t)e->n * 4));
+      SDR_CK(e, cudaMalloc(&e->d_magnitude, sdr_engine::RING_MAX * (size_t)e->n * 4));
       SDR_CK(e, cudaMalloc(&e->d_tracking, e->n));
       for (int i = 0; i < sdr_engine::RING_MAX; ++i) SDR_CK(e, cudaMalloc(&e->d_allowed[i], e->n));
       SDR_CK(e, cudaMalloc(&e->d_db_table, 128 * 4));
       // until now every block of every channel passed: the trackers are in `Tracking`
       // (SignalTracker.cc:104-145) if any block was seen, else in `NoSignal`
       SDR_CK(e, cudaMemsetAsync(e->d_tracking, e->seq > 0 ? 1 : 0, e->n, e->stream));
-      SDR_CK(e, cudaMemsetAsync(e->d_magnitude, 0, (size_t)e->n * 4, e->stream));
+      SDR_CK(e, cudaMemsetAsync(e->d_magnitude, 0, sdr_engine::RING_MAX * (size_t)e->n * 4, e->stream));
       int32_t table[128];
       for (int i = 1; i < 128; ++i) {  // DbfsCalculator.cc:60-68, host libm like the reference
         float db = 20 * log10f((float)i);
@@ -1031,8 +1044,9 @@ int run_squelch(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint64_t b
   q.threshold = e->d_threshold;
   q.gain_db = e->d_rx_gain;
   q.tracking = e->d_tracking;
+  // ring entry seq % RING_MAX: why three entries suffice behind an ingest ring, see run_iq_dump
   q.allowed = e->d_allowed[e->seq % (uint64_t)e->ring];
-  q.magnitude = e->d_magnitude;
+  q.magnitude = e->magnitude_of(e->seq);
   q.db_table = e->d_db_table;
   squelch_kernel<<<e->n, 128, 0, e->stream>>>(q);
   SDR_CK(e, cudaGetLastError());
@@ -1606,7 +1620,7 @@ int sdr_get_signal(sdr_engine *e, uint8_t *allowed, uint32_t *magnitude) {
   if (allowed)
     SDR_CK(e, cudaMemcpyAsync(allowed, e->d_allowed[(e->seq + (uint64_t)e->ring - 1) % (uint64_t)e->ring], e->n, cudaMemcpyDeviceToHost, e->stream));
   if (magnitude)
-    SDR_CK(e, cudaMemcpyAsync(magnitude, e->d_magnitude, (size_t)e->n * 4, cudaMemcpyDeviceToHost, e->stream));
+    SDR_CK(e, cudaMemcpyAsync(magnitude, e->magnitude_of(e->seq - 1), (size_t)e->n * 4, cudaMemcpyDeviceToHost, e->stream));
   SDR_CK(e, cudaStreamSynchronize(e->stream));
   return SDR_OK;
 }
@@ -1615,6 +1629,8 @@ int sdr_set_iq_dump(sdr_engine *e, uint32_t ch, int on) {
   if (!e || ch >= e->n) return SDR_E_ARG;
   if (e->dump_on[ch] != (uint8_t)(on != 0)) {
     e->dump_on[ch] = on != 0;
+    if (on) e->dump_count++;
+    else e->dump_count--;
     e->dump_dirty = true;
   }
   return SDR_OK;
@@ -1629,7 +1645,7 @@ int sdr_get_iq_dump(sdr_engine *e, uint32_t ch, int8_t *out, uint64_t capacity, 
   if (out && capacity < e->dump_bytes) return fail(e, SDR_E_ARG, "IQ dump buffer too small");
   SDR_CK(e, cudaSetDevice(e->device));
   if (out) {
-    SDR_CK(e, cudaMemcpyAsync(out, e->d_dump + (size_t)(it - e->dump_list.begin()) * e->max_bytes, e->dump_bytes,
+    SDR_CK(e, cudaMemcpyAsync(out, e->dump_of(e->seq - 1) + (size_t)(it - e->dump_list.begin()) * e->max_bytes, e->dump_bytes,
                               cudaMemcpyDeviceToHost, e->stream));
     SDR_CK(e, cudaStreamSynchronize(e->stream));
   }
@@ -1639,7 +1655,7 @@ int sdr_get_iq_dump(sdr_engine *e, uint32_t ch, int8_t *out, uint64_t capacity, 
 
 int sdr_iq_dump_device(sdr_engine *e, int8_t **rows, uint64_t *row_stride, uint32_t *n_rows) {
   if (!e) return SDR_E_ARG;
-  if (rows) *rows = e->d_dump;
+  if (rows) *rows = e->d_dump ? e->dump_of(e->seq ? e->seq - 1 : 0) : nullptr;  // the entry of the last call
   if (row_stride) *row_stride = e->max_bytes;
   if (n_rows) *n_rows = e->dump_bytes ? (uint32_t)e->dump_list.size() : 0;
   return SDR_OK;
@@ -1670,20 +1686,30 @@ struct sdr_ingest {
     uint8_t *h_iq = nullptr, *d_iq = nullptr;
     int16_t *h_pcm = nullptr;
     uint8_t *h_gate = nullptr;
+    uint32_t *h_magnitude = nullptr;
+    int8_t *h_dump = nullptr;    // [dump_cap][block_bytes], grown at commit time
+    uint32_t dump_cap = 0;
     cudaEvent_t ev_h2d = nullptr, ev_comp = nullptr, ev_done = nullptr;
     bool own_host = true;        // false: h_iq belongs to a bank's shared tick array
-    int16_t *pcm_dst = nullptr;  // where this tick's PCM was copied to (h_pcm, or a bank's shared array)
+    // where this tick's PCM, gate, magnitudes and dump rows were copied to: the slot's own arrays,
+    // or a bank's shared ones
+    int16_t *pcm_dst = nullptr;
+    uint8_t *gate_dst = nullptr;
+    uint32_t *mag_dst = nullptr;
+    int8_t *dump_dst = nullptr;
     uint32_t timestamp = 0;
     uint64_t bytes = 0;
-    bool gated = false, queued = false;
+    bool gated = false, queued = false;  // gated: the squelch ran for this tick
     std::vector<uint8_t> mode;
     std::vector<uint32_t> counts;
+    std::vector<uint32_t> dump_channels;  // the dumped channels, ascending; their rows are block_bytes apart
   };
   sdr_engine *e = nullptr;
   uint64_t block_bytes = 0;
   std::vector<Slot> slot;
   uint32_t head = 0, tail = 0, in_flight = 0;
   int prev = -1, prev2 = -1; // the slots of the last two ticks (see sdr_ingest_commit)
+  int retired = -1;          // the slot of the last retired tick
   cudaStream_t h2d = nullptr, d2h = nullptr;
   uint32_t last_timestamp = 0, short_blocks = 0;
   uint64_t ticks = 0;
@@ -1699,13 +1725,18 @@ int sdr_ingest_destroy(sdr_ingest *q) {
     if (s.own_host) cudaFreeHost(s.h_iq);
     cudaFreeHost(s.h_pcm);
     cudaFreeHost(s.h_gate);
+    cudaFreeHost(s.h_magnitude);
+    cudaFreeHost(s.h_dump);
     cudaFree(s.d_iq);
     if (s.ev_h2d) cudaEventDestroy(s.ev_h2d);
     if (s.ev_comp) cudaEventDestroy(s.ev_comp);
     if (s.ev_done) cudaEventDestroy(s.ev_done);
   }
   if (q->h2d) cudaStreamDestroy(q->h2d);
-  if (q->d2h) cudaStreamDestroy(q->d2h);
+  if (q->d2h) {
+    if (q->e->dump_reader == q->d2h) q->e->dump_reader = nullptr;
+    cudaStreamDestroy(q->d2h);
+  }
   delete q;
   return SDR_OK;
 }
@@ -1714,9 +1745,13 @@ int sdr_ingest_destroy(sdr_ingest *q) {
 
 namespace {
 // host_iq: null, or n_slots pointers to pinned [n_channels][block_bytes] arrays the slots use instead
-// of their own (a bank's shared tick arrays; then no per-slot PCM array is allocated either)
+// of their own (a bank's shared tick arrays; then no per-slot PCM, gate, magnitude or dump array is
+// allocated either)
 int ingest_create(sdr_engine *e, uint32_t n_slots, uint64_t block_bytes, uint8_t *const *host_iq, sdr_ingest **out);
-int ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t flags, int16_t *pcm_dst);
+// pcm_dst, gate_dst, mag_dst, dump_dst: null (the slot's own arrays), or where a bank gathers this
+// shard's PCM rows, gate, magnitudes and dump rows (dump rows block_bytes apart)
+int ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t flags, int16_t *pcm_dst,
+                  uint8_t *gate_dst, uint32_t *mag_dst, int8_t *dump_dst);
 }  // namespace
 
 extern "C" {
@@ -1749,6 +1784,7 @@ int ingest_create(sdr_engine *e, uint32_t n_slots, uint64_t block_bytes, uint8_t
   } while (0)
   SDR_CK_Q(cudaStreamCreateWithFlags(&q->h2d, cudaStreamNonBlocking));
   SDR_CK_Q(cudaStreamCreateWithFlags(&q->d2h, cudaStreamNonBlocking));
+  e->dump_reader = q->d2h;
   const size_t iq_bytes = (size_t)e->n * block_bytes, pcm_bytes = (size_t)e->n * (block_bytes / 64) * 2;
   for (uint32_t i = 0; i < n_slots; ++i) {
     sdr_ingest::Slot &s = q->slot[i];
@@ -1758,8 +1794,9 @@ int ingest_create(sdr_engine *e, uint32_t n_slots, uint64_t block_bytes, uint8_t
     } else {
       SDR_CK_Q(cudaHostAlloc(&s.h_iq, iq_bytes, cudaHostAllocDefault));
       SDR_CK_Q(cudaHostAlloc(&s.h_pcm, pcm_bytes, cudaHostAllocDefault));
+      SDR_CK_Q(cudaHostAlloc(&s.h_gate, e->n, cudaHostAllocDefault));
+      SDR_CK_Q(cudaHostAlloc(&s.h_magnitude, (size_t)e->n * 4, cudaHostAllocDefault));
     }
-    SDR_CK_Q(cudaHostAlloc(&s.h_gate, e->n, cudaHostAllocDefault));
     SDR_CK_Q(cudaMalloc(&s.d_iq, iq_bytes));
     SDR_CK_Q(cudaEventCreateWithFlags(&s.ev_h2d, cudaEventDisableTiming));
     SDR_CK_Q(cudaEventCreateWithFlags(&s.ev_comp, cudaEventDisableTiming));
@@ -1784,23 +1821,32 @@ int sdr_ingest_acquire(sdr_ingest *q, void **iq, uint64_t *channel_stride) {
 }
 
 int sdr_ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t flags) {
-  return ingest_commit(q, timestamp, bytes, flags, nullptr);
+  return ingest_commit(q, timestamp, bytes, flags, nullptr, nullptr, nullptr, nullptr);
 }
 
 }  // extern "C"
 
 namespace {
-int ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t flags, int16_t *pcm_dst) {
+int ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t flags, int16_t *pcm_dst,
+                  uint8_t *gate_dst, uint32_t *mag_dst, int8_t *dump_dst) {
   if (!q) return SDR_E_ARG;
   sdr_engine *e = q->e;
   sdr_ingest::Slot &s = q->slot[q->head];
   if (s.queued) return fail(e, SDR_E_FULL, "ingest ring full: retire a tick first");
   if (bytes == 0 || bytes % 64) return fail(e, SDR_E_ARG, "bytes_per_channel must be a positive multiple of 64");
+  SDR_CK(e, cudaSetDevice(e->device));
+  // the slot is free, so no copy of an earlier tick still lands in its dump array
+  if (!dump_dst && e->dump_count > s.dump_cap) {
+    cudaFreeHost(s.h_dump);
+    s.h_dump = nullptr;
+    s.dump_cap = 0;
+    SDR_CK(e, cudaHostAlloc(&s.h_dump, (size_t)e->dump_count * q->block_bytes, cudaHostAllocDefault));
+    s.dump_cap = e->dump_count;
+  }
   // DataConsumer::acceptData, DataConsumer.cc:232-246: clip to the buffer, count short blocks
   q->last_timestamp = timestamp;
   if (bytes > q->block_bytes) bytes = q->block_bytes;
   else if (bytes < q->block_bytes) q->short_blocks++;
-  SDR_CK(e, cudaSetDevice(e->device));
   if (bytes == q->block_bytes)
     SDR_CK(e, cudaMemcpyAsync(s.d_iq, s.h_iq, (size_t)e->n * bytes, cudaMemcpyHostToDevice, q->h2d));
   else
@@ -1819,9 +1865,21 @@ int ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t fl
   const size_t row = (size_t)(bytes / 64) * 2;
   s.pcm_dst = pcm_dst ? pcm_dst : s.h_pcm;
   SDR_CK(e, cudaMemcpy2DAsync(s.pcm_dst, row, e->pcm_of(e->seq - 1), e->pcm_stride * 2, row, e->n, cudaMemcpyDeviceToHost, q->d2h));
+  // the tick's signal reports and IQ dump, from the engine's ring entries of this call (run_iq_dump
+  // shows why they are not overwritten before these copies ran)
   s.gated = e->last_gated;
-  if (s.gated)
-    SDR_CK(e, cudaMemcpyAsync(s.h_gate, e->d_allowed[(e->seq + (uint64_t)e->ring - 1) % (uint64_t)e->ring], e->n, cudaMemcpyDeviceToHost, q->d2h));
+  s.gate_dst = gate_dst ? gate_dst : s.h_gate;
+  s.mag_dst = mag_dst ? mag_dst : s.h_magnitude;
+  if (s.gated) {
+    SDR_CK(e, cudaMemcpyAsync(s.gate_dst, e->d_allowed[(e->seq + (uint64_t)e->ring - 1) % (uint64_t)e->ring], e->n, cudaMemcpyDeviceToHost, q->d2h));
+    SDR_CK(e, cudaMemcpyAsync(s.mag_dst, e->magnitude_of(e->seq - 1), (size_t)e->n * 4, cudaMemcpyDeviceToHost, q->d2h));
+  }
+  s.dump_channels.clear();
+  if (e->dump_bytes) s.dump_channels = e->dump_list;
+  s.dump_dst = dump_dst ? dump_dst : s.h_dump;
+  if (!s.dump_channels.empty())
+    SDR_CK(e, cudaMemcpy2DAsync(s.dump_dst, q->block_bytes, e->dump_of(e->seq - 1), e->max_bytes, bytes,
+                                s.dump_channels.size(), cudaMemcpyDeviceToHost, q->d2h));
   SDR_CK(e, cudaEventRecord(s.ev_done, q->d2h));
   s.timestamp = timestamp;
   s.bytes = bytes;
@@ -1861,14 +1919,46 @@ int sdr_ingest_retire(sdr_ingest *q, uint32_t *timestamp, const int16_t **pcm, u
   SDR_CK(e, cudaEventSynchronize(s.ev_done));
   const uint32_t samples = (uint32_t)(s.bytes / 64);
   for (uint32_t ch = 0; ch < e->n; ++ch)
-    s.counts[ch] = (s.mode[ch] == SDR_MODE_NONE || (s.gated && !s.h_gate[ch])) ? 0 : samples;
+    s.counts[ch] = (s.mode[ch] == SDR_MODE_NONE || (s.gated && !s.gate_dst[ch])) ? 0 : samples;
   if (timestamp) *timestamp = s.timestamp;
   if (pcm) *pcm = s.pcm_dst;
   if (samples_per_row) *samples_per_row = samples;
   if (counts) *counts = s.counts.data();
   s.queued = false;
+  q->retired = (int)q->tail;
   q->tail = (q->tail + 1) % (uint32_t)q->slot.size();
   q->in_flight--;
+  return SDR_OK;
+}
+
+// the slot of the last retired tick, or null if there is none (or its slot was committed again)
+static const sdr_ingest::Slot *ingest_retired(const sdr_ingest *q) {
+  if (q->retired < 0 || q->slot[q->retired].queued) return nullptr;
+  return &q->slot[q->retired];
+}
+
+int sdr_ingest_retired_signal(const sdr_ingest *q, const uint8_t **allowed, const uint32_t **magnitude) {
+  if (!q) return SDR_E_ARG;
+  const sdr_ingest::Slot *s = ingest_retired(q);
+  if (!s) return fail(q->e, SDR_E_EMPTY, "no retired tick: retire one first");
+  if (!s->gated)
+    return fail(q->e, SDR_E_ARG, "the retired tick ran no squelch: set a threshold or enable signal reports before its commit");
+  if (allowed) *allowed = s->gate_dst;
+  if (magnitude) *magnitude = s->mag_dst;
+  return SDR_OK;
+}
+
+int sdr_ingest_retired_iq_dump(const sdr_ingest *q, const int8_t **rows, uint64_t *row_stride, uint64_t *n_bytes,
+                               const uint32_t **channels, uint32_t *n_rows) {
+  if (!q) return SDR_E_ARG;
+  const sdr_ingest::Slot *s = ingest_retired(q);
+  if (!s) return fail(q->e, SDR_E_EMPTY, "no retired tick: retire one first");
+  const bool any = !s->dump_channels.empty();
+  if (rows) *rows = any ? s->dump_dst : nullptr;
+  if (row_stride) *row_stride = q->block_bytes;
+  if (n_bytes) *n_bytes = s->bytes;
+  if (channels) *channels = any ? s->dump_channels.data() : nullptr;
+  if (n_rows) *n_rows = (uint32_t)s->dump_channels.size();
   return SDR_OK;
 }
 
@@ -1902,11 +1992,19 @@ struct sdr_bank {
   struct Slot {
     uint8_t *h_iq = nullptr;
     int16_t *h_pcm = nullptr;
+    uint8_t *h_allowed = nullptr;   // [n_channels], every shard's gate lands in its part
+    uint32_t *h_magnitude = nullptr;
+    int8_t *h_dump = nullptr;       // [dump_cap][block_bytes]: every shard's dump rows, in global channel order
+    uint32_t dump_cap = 0;
     std::vector<uint32_t> counts;
+    std::vector<uint32_t> dump_channels;  // global indices of the rows of h_dump
+    uint64_t bytes = 0;
+    bool gated = false;  // every shard ran the squelch for this tick
     bool queued = false;
   };
   std::vector<Slot> slot;
   uint32_t head = 0, tail = 0;
+  int retired = -1;  // the slot of the last retired tick
   std::string err;
 };
 
@@ -1934,6 +2032,9 @@ int sdr_bank_destroy(sdr_bank *b) {
   for (auto &s : b->slot) {
     cudaFreeHost(s.h_iq);
     cudaFreeHost(s.h_pcm);
+    cudaFreeHost(s.h_allowed);
+    cudaFreeHost(s.h_magnitude);
+    cudaFreeHost(s.h_dump);
   }
   delete b;
   return SDR_OK;
@@ -1959,10 +2060,12 @@ int sdr_bank_create(uint32_t n_channels, const int *devices, uint32_t n_devices,
   b->eng.assign(n_devices, nullptr);
   b->ing.assign(n_devices, nullptr);
   b->slot.resize(n_slots);
-  // the shared tick and PCM arrays: pinned for every device's context
+  // the shared tick, PCM, gate and magnitude arrays: pinned for every device's context
   for (auto &s : b->slot) {
     cudaError_t ce = cudaHostAlloc(&s.h_iq, (size_t)n_channels * block_bytes, cudaHostAllocPortable);
     if (ce == cudaSuccess) ce = cudaHostAlloc(&s.h_pcm, (size_t)n_channels * (block_bytes / 64) * 2, cudaHostAllocPortable);
+    if (ce == cudaSuccess) ce = cudaHostAlloc(&s.h_allowed, n_channels, cudaHostAllocPortable);
+    if (ce == cudaSuccess) ce = cudaHostAlloc(&s.h_magnitude, (size_t)n_channels * 4, cudaHostAllocPortable);
     if (ce != cudaSuccess) {
       bank_fail(nullptr, SDR_E_NOMEM, std::string("sdr_bank_create: pinned host memory: ") + cudaGetErrorString(ce));
       sdr_bank_destroy(b);
@@ -2044,6 +2147,24 @@ int sdr_bank_set_squelch_threshold(sdr_bank *b, uint32_t channel, int32_t thresh
   return sdr_set_squelch_threshold(b->eng[i], channel - b->first[i], threshold_dbfs);
 }
 
+int sdr_bank_set_receive_gain_db(sdr_bank *b, uint32_t channel, uint32_t gain_db) {
+  if (!b || channel >= b->n) return SDR_E_ARG;
+  const uint32_t i = bank_shard_of(b, channel);
+  return sdr_set_receive_gain_db(b->eng[i], channel - b->first[i], gain_db);
+}
+
+int sdr_bank_enable_signal_reports(sdr_bank *b, int on) {
+  if (!b) return SDR_E_ARG;
+  for (size_t i = 0; i < b->eng.size(); ++i) sdr_enable_signal_reports(b->eng[i], on);
+  return SDR_OK;
+}
+
+int sdr_bank_set_iq_dump(sdr_bank *b, uint32_t channel, int on) {
+  if (!b || channel >= b->n) return SDR_E_ARG;
+  const uint32_t i = bank_shard_of(b, channel);
+  return sdr_set_iq_dump(b->eng[i], channel - b->first[i], on);
+}
+
 int sdr_bank_acquire(sdr_bank *b, void **iq, uint64_t *channel_stride) {
   if (!b || !iq) return SDR_E_ARG;
   sdr_bank::Slot &s = b->slot[b->head];
@@ -2059,12 +2180,35 @@ int sdr_bank_commit(sdr_bank *b, uint32_t timestamp, uint64_t bytes, uint32_t fl
   if (s.queued) return bank_fail(b, SDR_E_FULL, "bank ring full: retire a tick first");
   if (bytes == 0 || bytes % 64) return bank_fail(b, SDR_E_ARG, "bytes_per_channel must be a positive multiple of 64");
   const uint64_t take = bytes > b->block_bytes ? b->block_bytes : bytes;  // clipped like DataConsumer.cc:232-246
-  for (size_t i = 0; i < b->eng.size(); ++i) {
-    // this device's slab of the shared PCM array, rows take / 64 samples apart
-    int16_t *dst = s.h_pcm + (size_t)b->first[i] * (take / 64);
-    const int rc = ingest_commit(b->ing[i], timestamp, bytes, flags, dst);
-    if (rc) return bank_fail_shard(b, rc, (uint32_t)i);
+  // the rows every shard will dump (its channels with the dump on); the slot is free, so nothing
+  // still copies into its dump array
+  uint64_t dump_total = 0;
+  for (size_t i = 0; i < b->eng.size(); ++i) dump_total += b->eng[i]->dump_count;
+  if (dump_total > s.dump_cap) {
+    cudaFreeHost(s.h_dump);
+    s.h_dump = nullptr;
+    s.dump_cap = 0;
+    const cudaError_t ce = cudaHostAlloc(&s.h_dump, dump_total * b->block_bytes, cudaHostAllocPortable);
+    if (ce != cudaSuccess)
+      return bank_fail(b, ce == cudaErrorMemoryAllocation ? SDR_E_NOMEM : SDR_E_CUDA,
+                       std::string("sdr_bank_commit: pinned host memory: ") + cudaGetErrorString(ce));
+    s.dump_cap = (uint32_t)dump_total;
   }
+  s.gated = true;
+  s.dump_channels.clear();
+  for (size_t i = 0; i < b->eng.size(); ++i) {
+    // this device's slabs of the shared arrays: PCM rows take / 64 samples apart, its gate and
+    // magnitudes, and its dump rows after those of the devices before it
+    int16_t *dst = s.h_pcm + (size_t)b->first[i] * (take / 64);
+    int8_t *dump_dst = s.h_dump ? s.h_dump + s.dump_channels.size() * b->block_bytes : nullptr;
+    const int rc = ingest_commit(b->ing[i], timestamp, bytes, flags, dst, s.h_allowed + b->first[i],
+                                 s.h_magnitude + b->first[i], dump_dst);
+    if (rc) return bank_fail_shard(b, rc, (uint32_t)i);
+    const sdr_ingest::Slot &t = b->ing[i]->slot[b->ing[i]->prev];  // the slot just committed
+    s.gated = s.gated && t.gated;
+    for (uint32_t ch : t.dump_channels) s.dump_channels.push_back(ch + b->first[i]);
+  }
+  s.bytes = take;
   s.queued = true;
   b->head = (b->head + 1) % (uint32_t)b->slot.size();
   return SDR_OK;
@@ -2087,7 +2231,39 @@ int sdr_bank_retire(sdr_bank *b, uint32_t *timestamp, const int16_t **pcm, uint3
   if (samples_per_row) *samples_per_row = samples;
   if (counts) *counts = s.counts.data();
   s.queued = false;
+  b->retired = (int)b->tail;
   b->tail = (b->tail + 1) % (uint32_t)b->slot.size();
+  return SDR_OK;
+}
+
+// the slot of the last retired tick, or null if there is none (or its slot was committed again)
+static const sdr_bank::Slot *bank_retired(const sdr_bank *b) {
+  if (b->retired < 0 || b->slot[b->retired].queued) return nullptr;
+  return &b->slot[b->retired];
+}
+
+int sdr_bank_retired_signal(sdr_bank *b, const uint8_t **allowed, const uint32_t **magnitude) {
+  if (!b) return SDR_E_ARG;
+  const sdr_bank::Slot *s = bank_retired(b);
+  if (!s) return bank_fail(b, SDR_E_EMPTY, "no retired tick: retire one first");
+  if (!s->gated)
+    return bank_fail(b, SDR_E_ARG, "the retired tick ran no squelch on every device: set a threshold or enable signal reports before its commit");
+  if (allowed) *allowed = s->h_allowed;
+  if (magnitude) *magnitude = s->h_magnitude;
+  return SDR_OK;
+}
+
+int sdr_bank_retired_iq_dump(sdr_bank *b, const int8_t **rows, uint64_t *row_stride, uint64_t *n_bytes,
+                             const uint32_t **channels, uint32_t *n_rows) {
+  if (!b) return SDR_E_ARG;
+  const sdr_bank::Slot *s = bank_retired(b);
+  if (!s) return bank_fail(b, SDR_E_EMPTY, "no retired tick: retire one first");
+  const bool any = !s->dump_channels.empty();
+  if (rows) *rows = any ? s->h_dump : nullptr;
+  if (row_stride) *row_stride = b->block_bytes;
+  if (n_bytes) *n_bytes = s->bytes;
+  if (channels) *channels = any ? s->dump_channels.data() : nullptr;
+  if (n_rows) *n_rows = (uint32_t)s->dump_channels.size();
   return SDR_OK;
 }
 

@@ -229,7 +229,9 @@ int sdr_filter_bank_create(int device, int kind, uint32_t n_rows, const float *t
       return fb_fail(nullptr, SDR_E_ARG, "n_taps and factor need a tile that does not fit in 48 KB of shared memory");
     }
   }
-  cudaError_t ce = cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking);
+  // a blocking stream: device-resident runs are ordered after the work the caller queued on the
+  // legacy default stream (where e.g. torch writes the input and zeroes the output by default)
+  cudaError_t ce = cudaStreamCreateWithFlags(&b->own_stream, cudaStreamDefault);
   if (ce != cudaSuccess) { delete b; return fb_fail(nullptr, SDR_E_CUDA, "cudaStreamCreate", ce); }
   b->stream = b->own_stream;
   std::vector<int32_t> q32(n_taps);
@@ -290,7 +292,7 @@ int sdr_filter_bank_create_iir(int device, uint32_t n_rows, const float *b_taps,
   if (ce == cudaSuccess) ce = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
   if (ce != cudaSuccess) { delete b; return fb_fail(nullptr, SDR_E_CUDA, "IIR bank: occupancy query", ce); }
   b->resident_lanes = (uint64_t)(per_sm > 0 ? per_sm : 1) * (uint64_t)sms * 32;
-  ce = cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking);
+  ce = cudaStreamCreateWithFlags(&b->own_stream, cudaStreamDefault);  // blocking, see sdr_filter_bank_create
   if (ce != cudaSuccess) { delete b; return fb_fail(nullptr, SDR_E_CUDA, "cudaStreamCreate", ce); }
   b->stream = b->own_stream;
   const size_t cbytes = (size_t)b->C * n_rows * 4;
