@@ -26,10 +26,12 @@
  *   IqDataProcessor::setSignalDetectThreshold              sdr_set_squelch_threshold
  *     (src_diags/IqDataProcessor.cc:284-295)
  *   radio_adjustableReceiveGainInDb (IqDataProcessor.cc:8) sdr_set_receive_gain_db
+ *   acceptIqData's block length, the rtlsdr read size      sdr_set_squelch_block_bytes,
+ *     (src_diags/Radio.cc: 32768)                           sdr_bank_set_squelch_block_bytes
  *   signal-state / signal-magnitude callbacks              sdr_enable_signal_reports,
- *     (src_diags/IqDataProcessor.cc:771-790)                sdr_get_signal (direct calls),
- *                                                           sdr_ingest_retired_signal (ring),
- *                                                           sdr_bank_retired_signal (bank)
+ *     (src_diags/IqDataProcessor.cc:771-790)                sdr_get_signal(_blocks) (direct calls),
+ *                                                           sdr_ingest_retired_signal(_blocks) (ring),
+ *                                                           sdr_bank_retired_signal(_blocks) (bank)
  *   IqDataProcessor::enableIqDump / disableIqDump          sdr_set_iq_dump, sdr_bank_set_iq_dump
  *     (src_diags/IqDataProcessor.cc:633-669)
  *   networkInterfacePtr->sendData(signedBufferPtr, n)      sdr_get_iq_dump / sdr_iq_dump_device,
@@ -117,8 +119,9 @@ int sdr_reset(sdr_engine *e, uint32_t channel, int kind);
  * demodulated only if its mean magnitude, in dBFS minus the tuner gain, reaches the
  * threshold, or did so on the previous block (one-block tail); a squelched channel
  * produces no PCM (counts[ch] = 0) and its demodulator state does not advance. The
- * default threshold of -200 dBFS never closes (IqDataProcessor.cc:41). The decision is
- * per sdr_accept_iq call, as the reference's is per acceptIqData call. */
+ * default threshold of -200 dBFS never closes (IqDataProcessor.cc:41). The reference decides
+ * once per acceptIqData call; the engine decides once per sdr_accept_iq call, or once per squelch
+ * block (sdr_set_squelch_block_bytes). */
 int sdr_set_squelch_threshold(sdr_engine *e, uint32_t channel, int32_t threshold_dbfs);
 int sdr_set_receive_gain_db(sdr_engine *e, uint32_t channel, uint32_t gain_db);
 /* Compute the signal state and mean magnitude of every call even while no threshold can
@@ -129,6 +132,23 @@ int sdr_enable_signal_reports(sdr_engine *e, int on);
  * ring in use this is the newest committed tick, not the retired one: see
  * sdr_ingest_retired_signal. */
 int sdr_get_signal(sdr_engine *e, uint8_t *allowed, uint32_t *magnitude);
+/* Squelch block: the length in bytes per channel of the block the squelch judges, standing for the
+ * reference's acceptIqData length (32768, the rtlsdr read size in Radio.cc). 0 (the default) = one
+ * decision per sdr_accept_iq call. Otherwise a multiple of 2048 within max_bytes_per_channel: a call
+ * of `bytes` is then judged as ceil(bytes / block_bytes) blocks, the last one possibly shorter, each
+ * as if it were its own acceptIqData call. Each block gets its own gate and magnitude, the tracker's
+ * one-block tail carries from block to block and call to call, and a closed block is not
+ * demodulated (its channel's state does not advance). The PCM of the open blocks is compacted: row
+ * ch holds their samples in block order from column 0, counts[ch] of them (each block's samples at
+ * its own length); what lies beyond is unspecified. The IQ dump still holds the whole call. The
+ * result equals that of feeding the same stream one block per call. Takes effect at the next call
+ * (under an ingest ring: at the next commit). SDR_E_ARG for any other value. */
+int sdr_set_squelch_block_bytes(sdr_engine *e, uint64_t block_bytes);
+/* Gates and mean magnitudes of every block of the last call, block-major [*n_blocks][n_channels]
+ * each; *n_blocks is 1 while the squelch block is 0. Any pointer may be NULL: with both arrays NULL
+ * this only reports *n_blocks, without synchronising. Fails like sdr_get_signal. With a squelch
+ * block set, sdr_get_signal returns the last block's row: what the reference's callbacks said last. */
+int sdr_get_signal_blocks(sdr_engine *e, uint8_t *allowed, uint32_t *magnitude, uint32_t *n_blocks);
 
 /* IQ dump (IqDataProcessor.cc:756-760): keep, for the channels it is enabled on, the block
  * of each sdr_accept_iq call as the reference hands it to UdpClient::sendData -- signed,
@@ -157,7 +177,8 @@ int sdr_accept_iq(sdr_engine *e, const void *iq, uint64_t bytes_per_channel,
                   uint64_t channel_stride, uint32_t flags);
 
 /* PCM of the last sdr_accept_iq: row ch holds counts[ch] samples (bytes/64, or 0
- * in mode None), rows are samples_per_row = bytes_per_channel/64 apart.
+ * in mode None or squelched; with a squelch block set, the open blocks' samples, compacted),
+ * rows are samples_per_row = bytes_per_channel/64 apart.
  * Synchronises. Either pointer may be NULL. */
 int sdr_get_pcm(sdr_engine *e, int16_t *pcm, uint32_t *counts);
 /* Device-resident PCM of the last call: [n_channels][*stride] int16. The engine alternates
@@ -202,6 +223,11 @@ int sdr_ingest_retire(sdr_ingest *q, uint32_t *timestamp, const int16_t **pcm, u
 /* Gate and mean magnitude of the last retired tick, [n_channels] each; either may be NULL.
  * SDR_E_ARG if that tick ran no squelch (no threshold that can close and reports off at its commit). */
 int sdr_ingest_retired_signal(const sdr_ingest *q, const uint8_t **allowed, const uint32_t **magnitude);
+/* Gates and mean magnitudes of every squelch block of the last retired tick, [*n_blocks][n_channels]
+ * each (sdr_set_squelch_block_bytes as it stood at the tick's commit; sdr_ingest_retired_signal
+ * returns the last row). Same codes and lifetimes as sdr_ingest_retired_signal. */
+int sdr_ingest_retired_signal_blocks(const sdr_ingest *q, const uint8_t **allowed, const uint32_t **magnitude,
+                                     uint32_t *n_blocks);
 /* IQ dump of the last retired tick: n_rows rows of *n_bytes (that tick's bytes_per_channel) signed, rotated
  * bytes, *row_stride apart, for channels[0..n_rows) in ascending order; n_rows = 0 if none was dumped. */
 int sdr_ingest_retired_iq_dump(const sdr_ingest *q, const int8_t **rows, uint64_t *row_stride, uint64_t *n_bytes,
@@ -237,6 +263,9 @@ int sdr_bank_set_receive_gain_db(sdr_bank *b, uint32_t channel, uint32_t gain_db
 int sdr_bank_set_iq_dump(sdr_bank *b, uint32_t channel, int on);
 /* sdr_enable_signal_reports on every shard */
 int sdr_bank_enable_signal_reports(sdr_bank *b, int on);
+/* sdr_set_squelch_block_bytes on every shard (a commit fails with SDR_E_ARG while the shards'
+ * settings would cut its tick into different numbers of blocks) */
+int sdr_bank_set_squelch_block_bytes(sdr_bank *b, uint64_t block_bytes);
 /* The next free tick array, [n_channels][*channel_stride] bytes of pinned host memory. */
 int sdr_bank_acquire(sdr_bank *b, void **iq, uint64_t *channel_stride);
 /* Queue the acquired tick on every device (flags: SDR_IQ_U8_OFFSET or SDR_IQ_S8_ROTATED). A tick
@@ -249,9 +278,12 @@ int sdr_bank_retire(sdr_bank *b, uint32_t *timestamp, const int16_t **pcm, uint3
 /* The signal reports and IQ dump of the tick the last sdr_bank_retire returned, gathered like its PCM
  * into pinned arrays of the slot (valid until the slot is acquired again); the rules and codes are
  * those of sdr_ingest_retired_signal / sdr_ingest_retired_iq_dump. The gate and magnitudes are
- * [n_channels]; SDR_E_ARG unless every shard ran the squelch for that tick. The dump rows are in
- * ascending global channel order across shards. */
+ * [n_channels] (with a squelch block set: the tick's last block); SDR_E_ARG unless every shard ran
+ * the squelch for that tick. The _blocks form returns every block, [*n_blocks][n_channels] in global
+ * channel order. The dump rows are in ascending global channel order across shards. */
 int sdr_bank_retired_signal(sdr_bank *b, const uint8_t **allowed, const uint32_t **magnitude);
+int sdr_bank_retired_signal_blocks(sdr_bank *b, const uint8_t **allowed, const uint32_t **magnitude,
+                                   uint32_t *n_blocks);
 int sdr_bank_retired_iq_dump(sdr_bank *b, const int8_t **rows, uint64_t *row_stride, uint64_t *n_bytes,
                              const uint32_t **channels, uint32_t *n_rows);
 /* Text of the last error on this bank (or of the last failed create if b is NULL). */

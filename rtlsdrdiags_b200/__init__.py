@@ -36,7 +36,9 @@ ABI_SYMBOLS = ["sdr_engine_create", "sdr_engine_destroy", "sdr_set_stream", "sdr
                "sdr_filter_bank_taps_q15", "sdr_filter_bank_launch_count", "sdr_filter_bank_last_error",
                "sdr_filter_bank_create_iir", "sdr_ingest_retired_signal", "sdr_ingest_retired_iq_dump",
                "sdr_bank_set_receive_gain_db", "sdr_bank_set_iq_dump", "sdr_bank_enable_signal_reports",
-               "sdr_bank_retired_signal", "sdr_bank_retired_iq_dump"]
+               "sdr_bank_retired_signal", "sdr_bank_retired_iq_dump", "sdr_set_squelch_block_bytes",
+               "sdr_get_signal_blocks", "sdr_ingest_retired_signal_blocks", "sdr_bank_set_squelch_block_bytes",
+               "sdr_bank_retired_signal_blocks"]
 
 
 class SdrError(RuntimeError):
@@ -76,6 +78,8 @@ def load_library(build_if_missing=True):
     L.sdr_set_receive_gain_db.argtypes = [vp, u32, u32]
     L.sdr_enable_signal_reports.argtypes = [vp, i32]
     L.sdr_get_signal.argtypes = [vp, vp, vp]
+    L.sdr_set_squelch_block_bytes.argtypes = [vp, u64]
+    L.sdr_get_signal_blocks.argtypes = [vp, vp, vp, C.POINTER(u32)]
     L.sdr_set_iq_dump.argtypes = [vp, u32, i32]
     L.sdr_get_iq_dump.argtypes = [vp, u32, vp, u64, C.POINTER(u64)]
     L.sdr_iq_dump_device.argtypes = [vp, C.POINTER(vp), C.POINTER(u64), C.POINTER(u32)]
@@ -87,6 +91,7 @@ def load_library(build_if_missing=True):
     L.sdr_ingest_retire.argtypes = [vp, C.POINTER(u32), C.POINTER(vp), C.POINTER(u32), C.POINTER(vp)]
     L.sdr_ingest_stats.argtypes = [vp, C.POINTER(u32), C.POINTER(u32), C.POINTER(u64), C.POINTER(u32)]
     L.sdr_ingest_retired_signal.argtypes = [vp, C.POINTER(vp), C.POINTER(vp)]
+    L.sdr_ingest_retired_signal_blocks.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(u32)]
     L.sdr_ingest_retired_iq_dump.argtypes = [vp, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64), C.POINTER(vp),
                                              C.POINTER(u32)]
     L.sdr_set_launch_shape.argtypes = [vp, i32, u32, u32]
@@ -116,6 +121,8 @@ def load_library(build_if_missing=True):
     L.sdr_bank_set_iq_dump.argtypes = [vp, u32, i32]
     L.sdr_bank_enable_signal_reports.argtypes = [vp, i32]
     L.sdr_bank_retired_signal.argtypes = [vp, C.POINTER(vp), C.POINTER(vp)]
+    L.sdr_bank_set_squelch_block_bytes.argtypes = [vp, u64]
+    L.sdr_bank_retired_signal_blocks.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(u32)]
     L.sdr_bank_retired_iq_dump.argtypes = [vp, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64), C.POINTER(vp),
                                            C.POINTER(u32)]
     L.sdr_bank_acquire.argtypes = [vp, C.POINTER(vp), C.POINTER(u64)]
@@ -150,6 +157,17 @@ def _retired_signal(fn, handle, n, ck):
     allowed = np.frombuffer((C.c_uint8 * n).from_address(a.value), dtype=np.uint8).astype(bool)
     mag = np.frombuffer((C.c_uint32 * n).from_address(m.value), dtype=np.uint32).copy()
     return allowed, mag
+
+
+def _retired_signal_blocks(fn, handle, n, ck):
+    """(allowed [n_blocks][n] bool, magnitude [n_blocks][n] uint32) through sdr_ingest_retired_signal_blocks /
+    sdr_bank_retired_signal_blocks."""
+    a, m, nb = C.c_void_p(), C.c_void_p(), C.c_uint32()
+    ck(fn(handle, C.byref(a), C.byref(m), C.byref(nb)))
+    cells = nb.value * n
+    allowed = np.frombuffer((C.c_uint8 * cells).from_address(a.value), dtype=np.uint8).astype(bool)
+    mag = np.frombuffer((C.c_uint32 * cells).from_address(m.value), dtype=np.uint32).copy()
+    return allowed.reshape(nb.value, n), mag.reshape(nb.value, n)
 
 
 def _retired_iq_dump(fn, handle, ck):
@@ -230,6 +248,22 @@ class Engine:
         a = np.empty(self.n, dtype=np.uint8)
         m = np.empty(self.n, dtype=np.uint32)
         self._ck(self.L.sdr_get_signal(self.h, a.ctypes.data_as(C.c_void_p), m.ctypes.data_as(C.c_void_p)))
+        return a.astype(bool), m
+
+    def set_squelch_block_bytes(self, block_bytes):
+        """Length in bytes of the block the squelch judges (the reference's acceptIqData length, 32768);
+        0 = one decision per call. From the next call on."""
+        self._ck(self.L.sdr_set_squelch_block_bytes(self.h, int(block_bytes)))
+
+    def get_signal_blocks(self):
+        """(allowed [n_blocks][n] bool, magnitude [n_blocks][n] uint32) of every squelch block of the last
+        accept. Synchronises."""
+        nb = C.c_uint32()
+        self._ck(self.L.sdr_get_signal_blocks(self.h, None, None, C.byref(nb)))
+        a = np.empty((nb.value, self.n), dtype=np.uint8)
+        m = np.empty((nb.value, self.n), dtype=np.uint32)
+        self._ck(self.L.sdr_get_signal_blocks(self.h, a.ctypes.data_as(C.c_void_p), m.ctypes.data_as(C.c_void_p),
+                                              C.byref(nb)))
         return a.astype(bool), m
 
     def set_iq_dump(self, channel, on=True):
@@ -397,6 +431,11 @@ class Ingest:
         signal-magnitude reports (IqDataProcessor.cc:771-790). Raises if that tick ran no squelch."""
         return _retired_signal(self.L.sdr_ingest_retired_signal, self.q, self.e.n, self.e._ck)
 
+    def retired_signal_blocks(self):
+        """(allowed [n_blocks][n] bool, magnitude [n_blocks][n] uint32) of every squelch block of the last
+        retired tick. Raises if that tick ran no squelch."""
+        return _retired_signal_blocks(self.L.sdr_ingest_retired_signal_blocks, self.q, self.e.n, self.e._ck)
+
     def retired_iq_dump(self):
         """{channel: int8 array} of the last retired tick's IQ dump (IqDataProcessor.cc:756-760)."""
         return _retired_iq_dump(self.L.sdr_ingest_retired_iq_dump, self.q, self.e._ck)
@@ -473,6 +512,15 @@ class Bank:
         """(allowed [n] bool, magnitude [n] uint32) of the last retired tick, gathered over all shards.
         Raises unless every shard ran the squelch for that tick."""
         return _retired_signal(self.L.sdr_bank_retired_signal, self.b, self.n, self._ck)
+
+    def set_squelch_block_bytes(self, block_bytes):
+        """Engine.set_squelch_block_bytes on every shard."""
+        self._ck(self.L.sdr_bank_set_squelch_block_bytes(self.b, int(block_bytes)))
+
+    def retired_signal_blocks(self):
+        """(allowed [n_blocks][n] bool, magnitude [n_blocks][n] uint32) of every squelch block of the last
+        retired tick, gathered over all shards."""
+        return _retired_signal_blocks(self.L.sdr_bank_retired_signal_blocks, self.b, self.n, self._ck)
 
     def retired_iq_dump(self):
         """{global channel: int8 array} of the last retired tick's IQ dump."""

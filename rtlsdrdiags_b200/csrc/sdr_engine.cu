@@ -74,7 +74,15 @@ struct sdr_engine {
   // dc_block_kernel's segmentation (0 = chosen per call) and its redo counter
   uint32_t dc_seg_count = 0, dc_warm_rows = 28;  // 896 steps: beyond the latest merge seen (807)
   uint32_t *d_counters = nullptr;
+  // Two counters. seq numbers the public calls: it picks the PCM buffer, the dump / gate /
+  // magnitude ring entries and the pace events. pass numbers the demodulation passes: it picks
+  // the scratch buffer and the ev_fir / ev_rec entry (par = pass % RING) and gives each pass its
+  // call_id. A call is one pass, or one pass per block while the squelch gates block by block
+  // (see accept_iq); with the squelch block at 0 the two counters are equal.
   uint64_t seq = 0;        // sdr_accept_iq calls so far
+  uint64_t pass = 0;       // demodulation passes so far
+  const uint8_t *pass_allowed = nullptr;  // gate row of the pass being queued, or null = all open
+  int16_t *pass_pcm = nullptr;            // where the pass being queued writes its PCM columns
   bool rec_pending = false;  // work on rec_stream that `stream` has not waited for yet
   // Mixed banks: the WBFM kernel (one long-lived CTA per SM that leaves issue slots, registers
   // and shared memory unused) runs on its own stream next to the other kinds' kernels
@@ -112,9 +120,18 @@ struct sdr_engine {
   bool squelch_dirty = false, squelch_armed = false, signal_reports = false;
   int32_t *d_threshold = nullptr;
   uint32_t *d_rx_gain = nullptr;
-  uint32_t *d_magnitude = nullptr;  // [RING_MAX][n], entry call % RING_MAX, like d_allowed
-  uint32_t *magnitude_of(uint64_t call) const { return d_magnitude + (size_t)(call % RING_MAX) * n; }
-  uint8_t *d_tracking = nullptr, *d_allowed[RING_MAX] = {};
+  // squelch block: bytes of the block the squelch judges (the reference's acceptIqData length),
+  // 0 = one decision per call
+  uint64_t squelch_block = 0;
+  uint32_t sig_rows = 1;  // block rows in each entry of d_allowed and d_magnitude
+  // gates and mean magnitudes, [RING_MAX][sig_rows][n]: entry call % RING_MAX, row = block
+  uint8_t *d_allowed = nullptr;
+  uint32_t *d_magnitude = nullptr;
+  uint8_t *allowed_of(uint64_t call) const { return d_allowed + (size_t)(call % RING_MAX) * sig_rows * n; }
+  uint32_t *magnitude_of(uint64_t call) const { return d_magnitude + (size_t)(call % RING_MAX) * sig_rows * n; }
+  uint32_t last_blocks = 1;       // blocks the last call's squelch judged (rows of its entry)
+  uint64_t last_block_bytes = 0;  // their length, the last one's excepted
+  uint8_t *d_tracking = nullptr;
   int32_t *d_db_table = nullptr;
   bool last_gated = false;  // the last accept ran the squelch kernel with the gate in force
   // blocks were accepted without the squelch kernel after d_tracking came to exist: every one of
@@ -209,7 +226,7 @@ float scale_of(int kind, float gain, int scaling) {
 // main stream waits for everything queued on rec_stream
 int join_streams(sdr_engine *e) {
   if (e->rec_pending) {
-    SDR_CK(e, cudaStreamWaitEvent(e->stream, e->ev_rec[(e->seq + (uint64_t)e->ring - 1) % (uint64_t)e->ring], 0));
+    SDR_CK(e, cudaStreamWaitEvent(e->stream, e->ev_rec[(e->pass + (uint64_t)e->ring - 1) % (uint64_t)e->ring], 0));
     e->rec_pending = false;
   }
   if (e->wb_pending) {
@@ -325,7 +342,7 @@ int launch_amssb(sdr_engine *e, int kind, const uint8_t *iq, uint64_t ch_stride,
   using T = AmSsbTile<SSB>;
   const uint32_t n_list = (uint32_t)e->list[kind].size();
   if (n_list == 0) return SDR_OK;
-  const int par = (int)(e->seq % (uint64_t)e->ring);
+  const int par = (int)(e->pass % (uint64_t)e->ring);
   const uint32_t n_tiles = (n_samples + TILE - 1) / TILE;
   if (!e->d_scratch[kind][par]) {
     // every buffer of the ring at the kind's first call: no allocation may fall into a later call
@@ -362,14 +379,14 @@ int launch_amssb(sdr_engine *e, int kind, const uint8_t *iq, uint64_t ch_stride,
   p.state_stride = (uint32_t)T::STATE_BYTES;
   p.scale = e->d_scale[kind];
   p.lsb = e->d_lsb;
-  p.pcm = e->pcm_of(e->seq);
+  p.pcm = e->pass_pcm;
   p.pcm_stride = e->pcm_stride;
   p.lut = nullptr;
   p.aux = (uint32_t)n_warps;
-  p.call_id = (uint32_t)(e->seq % 0x7fffffffull) + 1;
+  p.call_id = (uint32_t)(e->pass % 0x7fffffffull) + 1;
   p.scratch = e->d_scratch[kind][par];
-  p.allowed = e->last_gated ? e->d_allowed[par] : nullptr;
-  p.trace = e->d_trace ? e->d_trace + 4 * (e->seq % sdr_engine::TRACE_CALLS) : nullptr;
+  p.allowed = e->pass_allowed;
+  p.trace = e->d_trace ? e->d_trace + 4 * (e->pass % sdr_engine::TRACE_CALLS) : nullptr;
   const uint32_t grid = (uint32_t)((n_warps + 3) / 4);
   if (e->tile_loader == 0) {
     if (e->fir_ctas_per_sm == 6) amssb_fir_kernel<SSB, false, 2, false, 6><<<grid, 128, 4 * 2 * TILE_BYTES, e->stream>>>(p, e->tmap);
@@ -423,7 +440,7 @@ void dc_segments(const sdr_engine *e, uint32_t n_rows, uint32_t *seg_count, uint
 int launch_dc_block(sdr_engine *e, int kind, uint32_t n_samples) {
   const uint32_t n_list = (uint32_t)e->list[kind].size();
   if (n_list == 0) return SDR_OK;
-  const int par = (int)(e->seq % (uint64_t)e->ring);
+  const int par = (int)(e->pass % (uint64_t)e->ring);
   const int nreg = kind == SDR_KIND_SSB ? AmSsbTile<true>::NREG : AmSsbTile<false>::NREG;
   LaunchParams p = {};
   p.n_samples = n_samples;
@@ -432,12 +449,12 @@ int launch_dc_block(sdr_engine *e, int kind, uint32_t n_samples) {
   p.state = e->d_state[kind];
   p.state_stride = (uint32_t)state_bytes(kind);
   p.scale = e->d_scale[kind];
-  p.pcm = e->pcm_of(e->seq);
+  p.pcm = e->pass_pcm;
   p.pcm_stride = e->pcm_stride;
   p.aux = (uint32_t)nreg * 256;  // byte offset of the IIR tail in the state blob (after both carry buffers)
   p.scratch = e->d_scratch[kind][par];
-  p.allowed = e->last_gated ? e->d_allowed[par] : nullptr;
-  p.trace = e->d_trace ? e->d_trace + 4 * (e->seq % sdr_engine::TRACE_CALLS) + 2 : nullptr;
+  p.allowed = e->pass_allowed;
+  p.trace = e->d_trace ? e->d_trace + 4 * (e->pass % sdr_engine::TRACE_CALLS) + 2 : nullptr;
   dc_segments(e, (n_samples + TILE - 1) / TILE, &p.seg_count, &p.seg_rows);
   p.warm_rows = e->dc_warm_rows;
   p.counters = e->d_counters;
@@ -614,14 +631,14 @@ int launch_fm_tile(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint32_
   p.state_stride = (uint32_t)FmTile::STATE_BYTES;
   p.scale = e->d_scale[kind];
   p.lsb = e->d_lsb;
-  p.pcm = e->pcm_of(e->seq);
+  p.pcm = e->pass_pcm;
   p.pcm_stride = e->pcm_stride;
   p.lut = e->d_lut_fm;
   p.aux = (uint32_t)n_warps;
-  p.call_id = (uint32_t)(e->seq % 0x7fffffffull) + 1;
+  p.call_id = (uint32_t)(e->pass % 0x7fffffffull) + 1;
   p.tab = e->d_fm_tab;
   p.scratch = nullptr;
-  p.allowed = e->last_gated ? e->d_allowed[e->seq % (uint64_t)e->ring] : nullptr;
+  p.allowed = e->pass_allowed;
   const uint32_t grid = (uint32_t)((n_warps + G - 1) / G);
   static const int minb_env = getenv("SDR_FM_MIN_CTAS") ? atoi(getenv("SDR_FM_MIN_CTAS")) : 0;
   switch (minb_env) {
@@ -709,12 +726,12 @@ int launch_wbfm_tile3(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint
   p.state_stride = (uint32_t)WbTile::STATE_BYTES;
   p.scale = e->d_scale[kind];
   p.lsb = e->d_lsb;
-  p.pcm = e->pcm_of(e->seq);
+  p.pcm = e->pass_pcm;
   p.pcm_stride = e->pcm_stride;
   p.lut = e->d_lut_wbfm_half;
   p.aux = (uint32_t)std::min(workers, (int)T::REC_WARP);
   p.scratch = nullptr;
-  p.allowed = e->last_gated ? e->d_allowed[e->seq % (uint64_t)e->ring] : nullptr;
+  p.allowed = e->pass_allowed;
   p.tab = e->d_wb_tab;
   p.counters = e->wb_count ? e->d_counters : nullptr;  // one atomic per tile: only when somebody asked
   const uint32_t grid = (n_list + G - 1) / G;
@@ -770,7 +787,7 @@ int launch_wbfm_tile2(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint
   p.state_stride = (uint32_t)WbTile::STATE_BYTES;
   p.scale = e->d_scale[kind];
   p.lsb = e->d_lsb;
-  p.pcm = e->pcm_of(e->seq);
+  p.pcm = e->pass_pcm;
   p.pcm_stride = e->pcm_stride;
   p.lut = e->d_lut_wbfm_half;
   p.tab = e->d_wb_tab;
@@ -778,7 +795,7 @@ int launch_wbfm_tile2(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint
   static const int rec_env = getenv("SDR_WB_REC") ? atoi(getenv("SDR_WB_REC")) : -1;  // tuning override
   p.aux = (uint32_t)((rec_env >= 0 && rec_env <= (int)G) ? rec_env : std::min((int)G, (int)T::REC_WARP));
   p.scratch = nullptr;
-  p.allowed = e->last_gated ? e->d_allowed[e->seq % (uint64_t)e->ring] : nullptr;
+  p.allowed = e->pass_allowed;
   const uint32_t grid = (n_list + G - 1) / G;
   if (mma) {
     SDR_CK(e, cudaFuncSetAttribute(wbfm_tile2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -835,7 +852,7 @@ int launch_wbfm_tile4(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint
   p.state_stride = (uint32_t)WbTile::STATE_BYTES;
   p.scale = e->d_scale[kind];
   p.lsb = e->d_lsb;
-  p.pcm = e->pcm_of(e->seq);
+  p.pcm = e->pass_pcm;
   p.pcm_stride = e->pcm_stride;
   p.lut = e->d_lut_wbfm_half;
   p.aux = (uint32_t)rec;
@@ -843,7 +860,7 @@ int launch_wbfm_tile4(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint
   p.counters = e->d_counters;
   p.call_id = e->wb_count ? 1 : 0;  // the per-tile diagnostic counters: one atomic per tile, only when somebody asked
   p.scratch = nullptr;
-  p.allowed = e->last_gated ? e->d_allowed[e->seq % (uint64_t)e->ring] : nullptr;
+  p.allowed = e->pass_allowed;
   const uint32_t grid = (n_list + G - 1) / G;
   if (two) {
     SDR_CK(e, cudaFuncSetAttribute(wbfm_tile4_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -925,14 +942,14 @@ int launch_wbfm_tile(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint3
   p.state_stride = (uint32_t)T::STATE_BYTES;
   p.scale = e->d_scale[kind];
   p.lsb = e->d_lsb;
-  p.pcm = e->pcm_of(e->seq);
+  p.pcm = e->pass_pcm;
   p.pcm_stride = e->pcm_stride;
   p.lut = e->d_lut_wbfm;
   // workers allowed on the recurrence warp's scheduler (tunable: SDR_WB_S3)
   static const int s3_env = getenv("SDR_WB_S3") ? atoi(getenv("SDR_WB_S3")) : 4;
   p.aux = (uint32_t)s3_env;
   p.scratch = nullptr;
-  p.allowed = e->last_gated ? e->d_allowed[e->seq % (uint64_t)e->ring] : nullptr;
+  p.allowed = e->pass_allowed;
   SDR_CK(e, cudaFuncSetAttribute(wbfm_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   const uint32_t grid = (n_list + G - 1) / G;
   wbfm_tile_kernel<<<grid, 32 * T::warps_for((int)G, s3_env), smem, stream>>>(p);
@@ -979,7 +996,8 @@ int run_iq_dump(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint64_t b
   // d2h stream, after tick k's ev_comp and before its ev_done, and ingest_commit makes tick k+2's
   // work on `stream` wait for tick k's ev_done. Tick k+3, the next to write this entry, is queued on
   // `stream` after tick k+2, so its kernels start only once tick k's copies are over: three
-  // entries are enough however deep the ingest ring is.
+  // entries are enough however deep the ingest ring is. A call gated in block passes changes
+  // nothing here: its passes are all queued on `stream` (or wait on it) before tick k+1's work.
   d.out = e->dump_of(e->seq);
   d.out_stride = e->max_bytes;
   const uint64_t pieces = bytes / 16;
@@ -989,6 +1007,21 @@ int run_iq_dump(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint64_t b
   e->launches++;
   e->dump_bytes = bytes;
   return SDR_OK;
+}
+
+// Blocks the squelch judges in a call of `bytes` per channel at the current setting
+uint32_t squelch_blocks(const sdr_engine *e, uint64_t bytes) {
+  return e->squelch_block ? (uint32_t)((bytes + e->squelch_block - 1) / e->squelch_block) : 1;
+}
+
+// Samples channel ch produced in a call of `bytes` judged as n_blocks blocks of block_bytes
+// (the last one shorter), given the call's gates [n_blocks][pitch]: its open blocks' samples.
+uint32_t open_samples(const uint8_t *gate, uint64_t pitch, uint32_t ch, uint32_t n_blocks, uint64_t block_bytes,
+                      uint64_t bytes) {
+  uint64_t total = 0;
+  for (uint32_t k = 0; k < n_blocks; ++k)
+    if (gate[(size_t)k * pitch + ch]) total += (k + 1 == n_blocks ? bytes - (uint64_t)k * block_bytes : block_bytes) / 64;
+  return (uint32_t)total;
 }
 
 // Runs the squelch kernel when a threshold that can close is set (the gate is then in force)
@@ -1003,14 +1036,11 @@ int run_squelch(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint64_t b
     if ((armed || e->signal_reports) && !e->d_tracking) {
       SDR_CK(e, cudaMalloc(&e->d_threshold, (size_t)e->n * 4));
       SDR_CK(e, cudaMalloc(&e->d_rx_gain, (size_t)e->n * 4));
-      SDR_CK(e, cudaMalloc(&e->d_magnitude, sdr_engine::RING_MAX * (size_t)e->n * 4));
       SDR_CK(e, cudaMalloc(&e->d_tracking, e->n));
-      for (int i = 0; i < sdr_engine::RING_MAX; ++i) SDR_CK(e, cudaMalloc(&e->d_allowed[i], e->n));
       SDR_CK(e, cudaMalloc(&e->d_db_table, 128 * 4));
       // until now every block of every channel passed: the trackers are in `Tracking`
       // (SignalTracker.cc:104-145) if any block was seen, else in `NoSignal`
       SDR_CK(e, cudaMemsetAsync(e->d_tracking, e->seq > 0 ? 1 : 0, e->n, e->stream));
-      SDR_CK(e, cudaMemsetAsync(e->d_magnitude, 0, sdr_engine::RING_MAX * (size_t)e->n * 4, e->stream));
       int32_t table[128];
       for (int i = 1; i < 128; ++i) {  // DbfsCalculator.cc:60-68, host libm like the reference
         float db = 20 * log10f((float)i);
@@ -1036,16 +1066,37 @@ int run_squelch(sdr_engine *e, const uint8_t *iq, uint64_t ch_stride, uint64_t b
     SDR_CK(e, cudaMemsetAsync(e->d_tracking, 1, e->n, e->stream));
     e->tracking_stale = false;
   }
+  // gate and magnitude entries: one row per block of the longest call the setting allows
+  const uint32_t rows = std::max(e->sig_rows, squelch_blocks(e, e->max_bytes));
+  if (!e->d_allowed || rows > e->sig_rows) {
+    if (e->d_allowed) {  // queued recurrence kernels and read-back copies may still read the old entries
+      int rc = join_streams(e);
+      if (rc) return rc;
+      SDR_CK(e, cudaStreamSynchronize(e->stream));
+      if (e->dump_reader) SDR_CK(e, cudaStreamSynchronize(e->dump_reader));
+      cudaFree(e->d_allowed);
+      cudaFree(e->d_magnitude);
+      e->d_allowed = nullptr;
+      e->d_magnitude = nullptr;
+    }
+    e->sig_rows = rows;
+    const size_t cells = sdr_engine::RING_MAX * (size_t)rows * e->n;
+    SDR_CK(e, cudaMalloc(&e->d_allowed, cells));
+    SDR_CK(e, cudaMalloc(&e->d_magnitude, cells * 4));
+    SDR_CK(e, cudaMemsetAsync(e->d_magnitude, 0, cells * 4, e->stream));
+  }
   SquelchParams q;
   q.iq = iq;
   q.ch_stride = ch_stride;
   q.n_bytes = bytes;
+  q.block_bytes = e->squelch_block ? e->squelch_block : bytes;
+  q.n_channels = e->n;
   q.fmt = fmt;
   q.threshold = e->d_threshold;
   q.gain_db = e->d_rx_gain;
   q.tracking = e->d_tracking;
   // ring entry seq % RING_MAX: why three entries suffice behind an ingest ring, see run_iq_dump
-  q.allowed = e->d_allowed[e->seq % (uint64_t)e->ring];
+  q.allowed = e->allowed_of(e->seq);
   q.magnitude = e->magnitude_of(e->seq);
   q.db_table = e->d_db_table;
   squelch_kernel<<<e->n, 128, 0, e->stream>>>(q);
@@ -1252,7 +1303,7 @@ int sdr_engine_destroy(sdr_engine *e) {
   cudaFree(e->d_tracking);
   cudaFree(e->d_dump);
   cudaFree(e->d_dump_list);
-  for (int i = 0; i < sdr_engine::RING_MAX; ++i) cudaFree(e->d_allowed[i]);
+  cudaFree(e->d_allowed);
   cudaFree(e->d_db_table);
   cudaFree(e->d_lsb);
   cudaFree(e->d_lut_fm);
@@ -1460,6 +1511,8 @@ int sdr_debug_dc_redo_count(sdr_engine *e, uint32_t *count) {
 
 namespace {
 int accept_iq(sdr_engine *e, const void *iq, uint64_t bytes, uint64_t ch_stride, uint32_t flags);
+int wait_pass_slot(sdr_engine *e);
+int demodulate_pass(sdr_engine *e, const uint8_t *iq, uint64_t stride, uint32_t n_samples, int fmt, bool have_rec);
 int poisoned(sdr_engine *e) {
   e->err = "the engine is in a failed state after: " + e->poison_text;
   return SDR_E_CUDA;
@@ -1515,19 +1568,72 @@ int accept_iq(sdr_engine *e, const void *iq, uint64_t bytes, uint64_t ch_stride,
   if (e->seq % 4 == 0 && e->seq >= (uint64_t)sdr_engine::RUN_AHEAD)
     SDR_CK(e, cudaEventSynchronize(e->ev_pace[(int)(((e->seq - (uint64_t)sdr_engine::RUN_AHEAD) / 4) % (uint64_t)sdr_engine::PACE)]));
   const int fmt = (flags & SDR_IQ_S8_ROTATED) ? FMT_S8_ROTATED : FMT_U8_OFFSET_ROTATE;
-  const uint32_t n_samples = (uint32_t)(bytes / 2);
   const bool have_rec = !e->list[SDR_KIND_AM].empty() || !e->list[SDR_KIND_SSB].empty();
-  const int par = (int)(e->seq % (uint64_t)e->ring);
-  // scratch[par] and allowed[par] were last read by the recurrence kernels RING calls ago
-  // (usually long over: then no wait is queued at all)
+  // scratch[par] was last read by the recurrence kernels RING passes ago, and the gate entry this
+  // call's squelch writes by those of the call RING calls ago, whose passes are all at least RING
+  // passes old (usually long over: then no wait is queued at all)
   if (have_rec || e->squelch_armed || e->signal_reports || e->squelch_dirty) {
-    if (cudaEventQuery(e->ev_rec[par]) != cudaSuccess) {
-      (void)cudaGetLastError();  // "not ready" is an answer, not an error to be found later
-      SDR_CK(e, cudaStreamWaitEvent(e->stream, e->ev_rec[par], 0));
-    }
+    if ((rc = wait_pass_slot(e))) return rc;
   }
   if ((rc = run_iq_dump(e, dev_iq, dev_stride, bytes, fmt))) return rc;
   if ((rc = run_squelch(e, dev_iq, dev_stride, bytes, fmt))) return rc;
+  const uint32_t n_blocks = squelch_blocks(e, bytes);
+  e->last_blocks = n_blocks;
+  e->last_block_bytes = e->squelch_block ? e->squelch_block : bytes;
+  // While a gate is in force and the call holds several blocks, each block is its own pass: the
+  // same launches as a call of that block alone, reading the block's bytes, gated by its row and
+  // writing its PCM columns. Otherwise (reports only: every gate open) the call is one pass.
+  const bool split = e->last_gated && e->squelch_armed && n_blocks > 1;
+  const uint32_t passes = split ? n_blocks : 1;
+  const uint64_t pass_bytes = split ? e->squelch_block : bytes;
+  for (uint32_t k = 0; k < passes; ++k) {
+    const uint64_t off = (uint64_t)k * pass_bytes;
+    const uint64_t len = std::min(pass_bytes, bytes - off);
+    if (k > 0 && have_rec && (rc = wait_pass_slot(e))) return rc;
+    // Gate row k of this call's entry stays alive until its last reader, the recurrence kernel
+    // of pass k, is over: the entry is rewritten by the squelch of call seq + RING, which is
+    // queued after wait_pass_slot made `stream` wait for every pass at least RING passes old,
+    // and every pass of this call is that old by then (each call has at least one pass).
+    e->pass_allowed = e->last_gated ? e->allowed_of(e->seq) + (size_t)k * e->n : nullptr;
+    e->pass_pcm = e->pcm_of(e->seq) + off / 64;
+    if ((rc = demodulate_pass(e, dev_iq + off, dev_stride, (uint32_t)(len / 2), fmt, have_rec))) return rc;
+  }
+  if (split) {
+    // the open blocks' PCM to the front of each row, once every pass has written its columns
+    if ((rc = join_streams(e))) return rc;
+    CompactParams c;
+    c.pcm = e->pcm_of(e->seq);
+    c.pcm_stride = e->pcm_stride;
+    c.allowed = e->allowed_of(e->seq);
+    c.n_channels = e->n;
+    c.n_blocks = n_blocks;
+    c.block_samples = (uint32_t)(e->squelch_block / 64);
+    c.last_samples = (uint32_t)((bytes - (uint64_t)(n_blocks - 1) * e->squelch_block) / 64);
+    pcm_compact_kernel<<<e->n, 256, 0, e->stream>>>(c);
+    SDR_CK(e, cudaGetLastError());
+    e->launches++;
+  }
+  if (e->seq % 4 == 0) SDR_CK(e, cudaEventRecord(e->ev_pace[slot], e->stream));
+  e->seq++;
+  e->last_samples = (uint32_t)(bytes / 64);
+  return SDR_OK;
+}
+
+// `stream` waits for the recurrence kernels of the pass RING passes before the next one
+int wait_pass_slot(sdr_engine *e) {
+  const int par = (int)(e->pass % (uint64_t)e->ring);
+  if (cudaEventQuery(e->ev_rec[par]) != cudaSuccess) {
+    (void)cudaGetLastError();  // "not ready" is an answer, not an error to be found later
+    SDR_CK(e, cudaStreamWaitEvent(e->stream, e->ev_rec[par], 0));
+  }
+  return SDR_OK;
+}
+
+// One demodulation pass over n_samples of every channel from iq, into e->pass_pcm, gated by
+// e->pass_allowed.
+int demodulate_pass(sdr_engine *e, const uint8_t *iq, uint64_t stride, uint32_t n_samples, int fmt, bool have_rec) {
+  int rc;
+  const int par = (int)(e->pass % (uint64_t)e->ring);
   // WBFM first, and beside the others when there are others: its CTAs (one per SM for the whole
   // launch) take their place on every SM, the short-lived CTAs of the other kinds flow around them
   static const int wb_split_env = getenv("SDR_WB_SPLIT") ? atoi(getenv("SDR_WB_SPLIT")) : 1;
@@ -1536,26 +1642,24 @@ int accept_iq(sdr_engine *e, const void *iq, uint64_t bytes, uint64_t ch_stride,
   if (wb_beside) {
     SDR_CK(e, cudaEventRecord(e->ev_in, e->stream));
     SDR_CK(e, cudaStreamWaitEvent(e->wb_stream, e->ev_in, 0));
-    if ((rc = launch_wbfm_tile(e, dev_iq, dev_stride, n_samples, fmt, e->wb_stream))) return rc;
+    if ((rc = launch_wbfm_tile(e, iq, stride, n_samples, fmt, e->wb_stream))) return rc;
     SDR_CK(e, cudaEventRecord(e->ev_wb, e->wb_stream));
     e->wb_pending = true;
   }
-  if ((rc = launch_amssb<false>(e, SDR_KIND_AM, dev_iq, dev_stride, n_samples, fmt))) return rc;
-  if ((rc = launch_amssb<true>(e, SDR_KIND_SSB, dev_iq, dev_stride, n_samples, fmt))) return rc;
+  if ((rc = launch_amssb<false>(e, SDR_KIND_AM, iq, stride, n_samples, fmt))) return rc;
+  if ((rc = launch_amssb<true>(e, SDR_KIND_SSB, iq, stride, n_samples, fmt))) return rc;
   if (have_rec) {
     SDR_CK(e, cudaEventRecord(e->ev_fir[par], e->stream));
     SDR_CK(e, cudaStreamWaitEvent(e->rec_stream, e->ev_fir[par], 0));
     if ((rc = launch_dc_block(e, SDR_KIND_AM, n_samples))) return rc;
     if ((rc = launch_dc_block(e, SDR_KIND_SSB, n_samples))) return rc;
   }
-  // always recorded, so ev_rec[par] of the latest call orders after everything on rec_stream
+  // always recorded, so ev_rec[par] of the latest pass orders after everything on rec_stream
   SDR_CK(e, cudaEventRecord(e->ev_rec[par], e->rec_stream));
   e->rec_pending = true;
-  if ((rc = launch_fm_tile(e, dev_iq, dev_stride, n_samples, fmt))) return rc;
-  if (!wb_beside && (rc = launch_wbfm_tile(e, dev_iq, dev_stride, n_samples, fmt, e->stream))) return rc;
-  if (e->seq % 4 == 0) SDR_CK(e, cudaEventRecord(e->ev_pace[slot], e->stream));
-  e->seq++;
-  e->last_samples = (uint32_t)(bytes / 64);
+  if ((rc = launch_fm_tile(e, iq, stride, n_samples, fmt))) return rc;
+  if (!wb_beside && (rc = launch_wbfm_tile(e, iq, stride, n_samples, fmt, e->stream))) return rc;
+  e->pass++;
   return SDR_OK;
 }
 }  // namespace
@@ -1575,13 +1679,16 @@ int sdr_get_pcm(sdr_engine *e, int16_t *pcm, uint32_t *counts) {
                                 (size_t)e->last_samples * 2, e->n, cudaMemcpyDeviceToHost, e->stream));
   std::vector<uint8_t> gate;
   if (counts && e->last_gated && e->seq > 0) {
-    gate.resize(e->n);
-    SDR_CK(e, cudaMemcpyAsync(gate.data(), e->d_allowed[(e->seq + (uint64_t)e->ring - 1) % (uint64_t)e->ring], e->n, cudaMemcpyDeviceToHost, e->stream));
+    gate.resize((size_t)e->last_blocks * e->n);
+    SDR_CK(e, cudaMemcpyAsync(gate.data(), e->allowed_of(e->seq - 1), gate.size(), cudaMemcpyDeviceToHost, e->stream));
   }
   SDR_CK(e, cudaStreamSynchronize(e->stream));
   if (counts)
     for (uint32_t ch = 0; ch < e->n; ++ch)
-      counts[ch] = (e->mode[ch] == SDR_MODE_NONE || (!gate.empty() && !gate[ch])) ? 0 : e->last_samples;
+      counts[ch] = e->mode[ch] == SDR_MODE_NONE ? 0
+                   : gate.empty() ? e->last_samples
+                                  : open_samples(gate.data(), e->n, ch, e->last_blocks, e->last_block_bytes,
+                                                 (uint64_t)e->last_samples * 64);
   return SDR_OK;
 }
 
@@ -1617,10 +1724,33 @@ int sdr_get_signal(sdr_engine *e, uint8_t *allowed, uint32_t *magnitude) {
   if (!e) return SDR_E_ARG;
   if (!e->last_gated || e->seq == 0) return fail(e, SDR_E_ARG, "no squelch result: set a threshold or enable signal reports first");
   SDR_CK(e, cudaSetDevice(e->device));
+  const size_t last = (size_t)(e->last_blocks - 1) * e->n;  // the last block's row
   if (allowed)
-    SDR_CK(e, cudaMemcpyAsync(allowed, e->d_allowed[(e->seq + (uint64_t)e->ring - 1) % (uint64_t)e->ring], e->n, cudaMemcpyDeviceToHost, e->stream));
+    SDR_CK(e, cudaMemcpyAsync(allowed, e->allowed_of(e->seq - 1) + last, e->n, cudaMemcpyDeviceToHost, e->stream));
   if (magnitude)
-    SDR_CK(e, cudaMemcpyAsync(magnitude, e->magnitude_of(e->seq - 1), (size_t)e->n * 4, cudaMemcpyDeviceToHost, e->stream));
+    SDR_CK(e, cudaMemcpyAsync(magnitude, e->magnitude_of(e->seq - 1) + last, (size_t)e->n * 4, cudaMemcpyDeviceToHost, e->stream));
+  SDR_CK(e, cudaStreamSynchronize(e->stream));
+  return SDR_OK;
+}
+
+int sdr_set_squelch_block_bytes(sdr_engine *e, uint64_t block_bytes) {
+  if (!e) return SDR_E_ARG;
+  if (block_bytes % 2048 || block_bytes > e->max_bytes)
+    return fail(e, SDR_E_ARG, "squelch block must be 0 or a multiple of 2048 within max_bytes_per_channel");
+  e->squelch_block = block_bytes;
+  return SDR_OK;
+}
+
+int sdr_get_signal_blocks(sdr_engine *e, uint8_t *allowed, uint32_t *magnitude, uint32_t *n_blocks) {
+  if (!e) return SDR_E_ARG;
+  if (!e->last_gated || e->seq == 0) return fail(e, SDR_E_ARG, "no squelch result: set a threshold or enable signal reports first");
+  if (n_blocks) *n_blocks = e->last_blocks;
+  if (!allowed && !magnitude) return SDR_OK;
+  SDR_CK(e, cudaSetDevice(e->device));
+  const size_t cells = (size_t)e->last_blocks * e->n;
+  if (allowed) SDR_CK(e, cudaMemcpyAsync(allowed, e->allowed_of(e->seq - 1), cells, cudaMemcpyDeviceToHost, e->stream));
+  if (magnitude)
+    SDR_CK(e, cudaMemcpyAsync(magnitude, e->magnitude_of(e->seq - 1), cells * 4, cudaMemcpyDeviceToHost, e->stream));
   SDR_CK(e, cudaStreamSynchronize(e->stream));
   return SDR_OK;
 }
@@ -1689,6 +1819,7 @@ struct sdr_ingest {
     uint32_t *h_magnitude = nullptr;
     int8_t *h_dump = nullptr;    // [dump_cap][block_bytes], grown at commit time
     uint32_t dump_cap = 0;
+    uint32_t sig_cap = 1;        // block rows h_gate and h_magnitude hold, grown at commit time
     cudaEvent_t ev_h2d = nullptr, ev_comp = nullptr, ev_done = nullptr;
     bool own_host = true;        // false: h_iq belongs to a bank's shared tick array
     // where this tick's PCM, gate, magnitudes and dump rows were copied to: the slot's own arrays,
@@ -1699,6 +1830,10 @@ struct sdr_ingest {
     int8_t *dump_dst = nullptr;
     uint32_t timestamp = 0;
     uint64_t bytes = 0;
+    // the tick's squelch blocks: n_blocks rows of gates and magnitudes, sig_pitch channels apart at
+    // gate_dst / mag_dst, for blocks of sig_block bytes (the last one shorter)
+    uint32_t n_blocks = 1;
+    uint64_t sig_pitch = 0, sig_block = 0;
     bool gated = false, queued = false;  // gated: the squelch ran for this tick
     std::vector<uint8_t> mode;
     std::vector<uint32_t> counts;
@@ -1749,9 +1884,10 @@ namespace {
 // allocated either)
 int ingest_create(sdr_engine *e, uint32_t n_slots, uint64_t block_bytes, uint8_t *const *host_iq, sdr_ingest **out);
 // pcm_dst, gate_dst, mag_dst, dump_dst: null (the slot's own arrays), or where a bank gathers this
-// shard's PCM rows, gate, magnitudes and dump rows (dump rows block_bytes apart)
+// shard's PCM rows, gates, magnitudes and dump rows (block rows of gates and magnitudes sig_pitch
+// channels apart, dump rows block_bytes apart)
 int ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t flags, int16_t *pcm_dst,
-                  uint8_t *gate_dst, uint32_t *mag_dst, int8_t *dump_dst);
+                  uint8_t *gate_dst, uint32_t *mag_dst, uint64_t sig_pitch, int8_t *dump_dst);
 }  // namespace
 
 extern "C" {
@@ -1821,14 +1957,14 @@ int sdr_ingest_acquire(sdr_ingest *q, void **iq, uint64_t *channel_stride) {
 }
 
 int sdr_ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t flags) {
-  return ingest_commit(q, timestamp, bytes, flags, nullptr, nullptr, nullptr, nullptr);
+  return ingest_commit(q, timestamp, bytes, flags, nullptr, nullptr, nullptr, 0, nullptr);
 }
 
 }  // extern "C"
 
 namespace {
 int ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t flags, int16_t *pcm_dst,
-                  uint8_t *gate_dst, uint32_t *mag_dst, int8_t *dump_dst) {
+                  uint8_t *gate_dst, uint32_t *mag_dst, uint64_t sig_pitch, int8_t *dump_dst) {
   if (!q) return SDR_E_ARG;
   sdr_engine *e = q->e;
   sdr_ingest::Slot &s = q->slot[q->head];
@@ -1842,6 +1978,18 @@ int ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t fl
     s.dump_cap = 0;
     SDR_CK(e, cudaHostAlloc(&s.h_dump, (size_t)e->dump_count * q->block_bytes, cudaHostAllocDefault));
     s.dump_cap = e->dump_count;
+  }
+  const uint64_t take = bytes > q->block_bytes ? q->block_bytes : bytes;
+  const uint32_t n_blocks = squelch_blocks(e, take);
+  if (!gate_dst && n_blocks > s.sig_cap) {  // likewise for the gate and magnitude rows
+    cudaFreeHost(s.h_gate);
+    cudaFreeHost(s.h_magnitude);
+    s.h_gate = nullptr;
+    s.h_magnitude = nullptr;
+    s.sig_cap = 0;
+    SDR_CK(e, cudaHostAlloc(&s.h_gate, (size_t)n_blocks * e->n, cudaHostAllocDefault));
+    SDR_CK(e, cudaHostAlloc(&s.h_magnitude, (size_t)n_blocks * e->n * 4, cudaHostAllocDefault));
+    s.sig_cap = n_blocks;
   }
   // DataConsumer::acceptData, DataConsumer.cc:232-246: clip to the buffer, count short blocks
   q->last_timestamp = timestamp;
@@ -1870,9 +2018,14 @@ int ingest_commit(sdr_ingest *q, uint32_t timestamp, uint64_t bytes, uint32_t fl
   s.gated = e->last_gated;
   s.gate_dst = gate_dst ? gate_dst : s.h_gate;
   s.mag_dst = mag_dst ? mag_dst : s.h_magnitude;
-  if (s.gated) {
-    SDR_CK(e, cudaMemcpyAsync(s.gate_dst, e->d_allowed[(e->seq + (uint64_t)e->ring - 1) % (uint64_t)e->ring], e->n, cudaMemcpyDeviceToHost, q->d2h));
-    SDR_CK(e, cudaMemcpyAsync(s.mag_dst, e->magnitude_of(e->seq - 1), (size_t)e->n * 4, cudaMemcpyDeviceToHost, q->d2h));
+  s.sig_pitch = gate_dst ? sig_pitch : e->n;
+  s.n_blocks = e->last_blocks;
+  s.sig_block = e->last_block_bytes;
+  if (s.gated) {  // every block row of the entry, one 2D copy each
+    SDR_CK(e, cudaMemcpy2DAsync(s.gate_dst, s.sig_pitch, e->allowed_of(e->seq - 1), e->n, e->n, s.n_blocks,
+                                cudaMemcpyDeviceToHost, q->d2h));
+    SDR_CK(e, cudaMemcpy2DAsync(s.mag_dst, s.sig_pitch * 4, e->magnitude_of(e->seq - 1), (size_t)e->n * 4,
+                                (size_t)e->n * 4, s.n_blocks, cudaMemcpyDeviceToHost, q->d2h));
   }
   s.dump_channels.clear();
   if (e->dump_bytes) s.dump_channels = e->dump_list;
@@ -1919,7 +2072,9 @@ int sdr_ingest_retire(sdr_ingest *q, uint32_t *timestamp, const int16_t **pcm, u
   SDR_CK(e, cudaEventSynchronize(s.ev_done));
   const uint32_t samples = (uint32_t)(s.bytes / 64);
   for (uint32_t ch = 0; ch < e->n; ++ch)
-    s.counts[ch] = (s.mode[ch] == SDR_MODE_NONE || (s.gated && !s.gate_dst[ch])) ? 0 : samples;
+    s.counts[ch] = s.mode[ch] == SDR_MODE_NONE ? 0
+                   : !s.gated ? samples
+                              : open_samples(s.gate_dst, s.sig_pitch, ch, s.n_blocks, s.sig_block, s.bytes);
   if (timestamp) *timestamp = s.timestamp;
   if (pcm) *pcm = s.pcm_dst;
   if (samples_per_row) *samples_per_row = samples;
@@ -1943,8 +2098,22 @@ int sdr_ingest_retired_signal(const sdr_ingest *q, const uint8_t **allowed, cons
   if (!s) return fail(q->e, SDR_E_EMPTY, "no retired tick: retire one first");
   if (!s->gated)
     return fail(q->e, SDR_E_ARG, "the retired tick ran no squelch: set a threshold or enable signal reports before its commit");
+  const size_t last = (size_t)(s->n_blocks - 1) * s->sig_pitch;  // the last block's row
+  if (allowed) *allowed = s->gate_dst + last;
+  if (magnitude) *magnitude = s->mag_dst + last;
+  return SDR_OK;
+}
+
+int sdr_ingest_retired_signal_blocks(const sdr_ingest *q, const uint8_t **allowed, const uint32_t **magnitude,
+                                     uint32_t *n_blocks) {
+  if (!q) return SDR_E_ARG;
+  const sdr_ingest::Slot *s = ingest_retired(q);
+  if (!s) return fail(q->e, SDR_E_EMPTY, "no retired tick: retire one first");
+  if (!s->gated)
+    return fail(q->e, SDR_E_ARG, "the retired tick ran no squelch: set a threshold or enable signal reports before its commit");
   if (allowed) *allowed = s->gate_dst;
   if (magnitude) *magnitude = s->mag_dst;
+  if (n_blocks) *n_blocks = s->n_blocks;
   return SDR_OK;
 }
 
@@ -1992,8 +2161,10 @@ struct sdr_bank {
   struct Slot {
     uint8_t *h_iq = nullptr;
     int16_t *h_pcm = nullptr;
-    uint8_t *h_allowed = nullptr;   // [n_channels], every shard's gate lands in its part
+    // [sig_cap][n_channels]: block row k of every shard's gates and magnitudes lands in its columns
+    uint8_t *h_allowed = nullptr;
     uint32_t *h_magnitude = nullptr;
+    uint32_t sig_cap = 1, n_blocks = 1;
     int8_t *h_dump = nullptr;       // [dump_cap][block_bytes]: every shard's dump rows, in global channel order
     uint32_t dump_cap = 0;
     std::vector<uint32_t> counts;
@@ -2159,6 +2330,15 @@ int sdr_bank_enable_signal_reports(sdr_bank *b, int on) {
   return SDR_OK;
 }
 
+int sdr_bank_set_squelch_block_bytes(sdr_bank *b, uint64_t block_bytes) {
+  if (!b) return SDR_E_ARG;
+  for (size_t i = 0; i < b->eng.size(); ++i) {
+    const int rc = sdr_set_squelch_block_bytes(b->eng[i], block_bytes);
+    if (rc) return bank_fail_shard(b, rc, (uint32_t)i);
+  }
+  return SDR_OK;
+}
+
 int sdr_bank_set_iq_dump(sdr_bank *b, uint32_t channel, int on) {
   if (!b || channel >= b->n) return SDR_E_ARG;
   const uint32_t i = bank_shard_of(b, channel);
@@ -2194,6 +2374,26 @@ int sdr_bank_commit(sdr_bank *b, uint32_t timestamp, uint64_t bytes, uint32_t fl
                        std::string("sdr_bank_commit: pinned host memory: ") + cudaGetErrorString(ce));
     s.dump_cap = (uint32_t)dump_total;
   }
+  // the squelch blocks of this tick, the same on every shard; the gate and magnitude rows grow like
+  // the dump array
+  const uint32_t n_blocks = squelch_blocks(b->eng[0], take);
+  for (size_t i = 1; i < b->eng.size(); ++i)
+    if (squelch_blocks(b->eng[i], take) != n_blocks)
+      return bank_fail(b, SDR_E_ARG, "sdr_bank_commit: the shards' squelch blocks differ: set them with sdr_bank_set_squelch_block_bytes");
+  if (n_blocks > s.sig_cap) {
+    cudaFreeHost(s.h_allowed);
+    cudaFreeHost(s.h_magnitude);
+    s.h_allowed = nullptr;
+    s.h_magnitude = nullptr;
+    s.sig_cap = 0;
+    cudaError_t ce = cudaHostAlloc(&s.h_allowed, (size_t)n_blocks * b->n, cudaHostAllocPortable);
+    if (ce == cudaSuccess) ce = cudaHostAlloc(&s.h_magnitude, (size_t)n_blocks * b->n * 4, cudaHostAllocPortable);
+    if (ce != cudaSuccess)
+      return bank_fail(b, ce == cudaErrorMemoryAllocation ? SDR_E_NOMEM : SDR_E_CUDA,
+                       std::string("sdr_bank_commit: pinned host memory: ") + cudaGetErrorString(ce));
+    s.sig_cap = n_blocks;
+  }
+  s.n_blocks = n_blocks;
   s.gated = true;
   s.dump_channels.clear();
   for (size_t i = 0; i < b->eng.size(); ++i) {
@@ -2202,7 +2402,7 @@ int sdr_bank_commit(sdr_bank *b, uint32_t timestamp, uint64_t bytes, uint32_t fl
     int16_t *dst = s.h_pcm + (size_t)b->first[i] * (take / 64);
     int8_t *dump_dst = s.h_dump ? s.h_dump + s.dump_channels.size() * b->block_bytes : nullptr;
     const int rc = ingest_commit(b->ing[i], timestamp, bytes, flags, dst, s.h_allowed + b->first[i],
-                                 s.h_magnitude + b->first[i], dump_dst);
+                                 s.h_magnitude + b->first[i], b->n, dump_dst);
     if (rc) return bank_fail_shard(b, rc, (uint32_t)i);
     const sdr_ingest::Slot &t = b->ing[i]->slot[b->ing[i]->prev];  // the slot just committed
     s.gated = s.gated && t.gated;
@@ -2248,8 +2448,22 @@ int sdr_bank_retired_signal(sdr_bank *b, const uint8_t **allowed, const uint32_t
   if (!s) return bank_fail(b, SDR_E_EMPTY, "no retired tick: retire one first");
   if (!s->gated)
     return bank_fail(b, SDR_E_ARG, "the retired tick ran no squelch on every device: set a threshold or enable signal reports before its commit");
+  const size_t last = (size_t)(s->n_blocks - 1) * b->n;  // the last block's row
+  if (allowed) *allowed = s->h_allowed + last;
+  if (magnitude) *magnitude = s->h_magnitude + last;
+  return SDR_OK;
+}
+
+int sdr_bank_retired_signal_blocks(sdr_bank *b, const uint8_t **allowed, const uint32_t **magnitude,
+                                   uint32_t *n_blocks) {
+  if (!b) return SDR_E_ARG;
+  const sdr_bank::Slot *s = bank_retired(b);
+  if (!s) return bank_fail(b, SDR_E_EMPTY, "no retired tick: retire one first");
+  if (!s->gated)
+    return bank_fail(b, SDR_E_ARG, "the retired tick ran no squelch on every device: set a threshold or enable signal reports before its commit");
   if (allowed) *allowed = s->h_allowed;
   if (magnitude) *magnitude = s->h_magnitude;
+  if (n_blocks) *n_blocks = s->n_blocks;
   return SDR_OK;
 }
 

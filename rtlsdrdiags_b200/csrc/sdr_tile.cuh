@@ -1835,18 +1835,22 @@ __global__ void __launch_bounds__(256) iq_dump_kernel(const __grid_constant__ Du
 // magnitude estimate over the block (SignalDetector.cc:205-273), dBFS through the 7-bit
 // table (DbfsCalculator.cc:111-147), threshold, two-state tracker with a one-block tail
 // (SignalTracker.cc:104-145). One CTA per channel; runs before the demodulation kernels
-// when a threshold that can close is set or signal reports are wanted.
+// when a threshold that can close is set or signal reports are wanted. The call's bytes are
+// judged as blocks of block_bytes (the last one may be shorter), each as its own acceptIqData
+// call would be; the tracker steps from one block to the next.
 // ---------------------------------------------------------------------------
 struct SquelchParams {
   const uint8_t *iq;
   uint64_t ch_stride;
   uint64_t n_bytes;
+  uint64_t block_bytes;       // bytes per judged block (n_bytes: one decision for the call)
+  uint32_t n_channels;        // row length of allowed / magnitude
   int fmt;
   const int32_t *threshold;   // [n_channels] dBFS
   const uint32_t *gain_db;    // [n_channels] tuner gain (radio_adjustableReceiveGainInDb)
-  uint8_t *tracking;          // [n_channels] SignalTracker state, carried across calls
-  uint8_t *allowed;           // [n_channels] out: gate of this call
-  uint32_t *magnitude;        // [n_channels] out: mean magnitude of this call's block
+  uint8_t *tracking;          // [n_channels] SignalTracker state, carried across blocks and calls
+  uint8_t *allowed;           // [n_blocks][n_channels] out: gate of each block
+  uint32_t *magnitude;        // [n_blocks][n_channels] out: mean magnitude of each block
   const int32_t *db_table;    // [128] (int32_t)(20 log10f(i)), built by the host libm
 };
 
@@ -1854,38 +1858,80 @@ __global__ void __launch_bounds__(128) squelch_kernel(const SquelchParams q) {
   const uint32_t ch = blockIdx.x;
   const uint8_t *src = q.iq + (uint64_t)ch * q.ch_stride;
   const uint32_t flip = q.fmt == FMT_U8_OFFSET_ROTATE ? 0x80808080u : 0u;  // the rotation does not change |.|
-  unsigned long long sum = 0;
-  for (uint64_t c = threadIdx.x; c < q.n_bytes / 16; c += blockDim.x) {
-    const u32x4 v = ld_stream_u4(src + 16 * c);
-    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-    uint32_t part = 0;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const uint32_t a = __vabs4(w[i] ^ flip);          // |i|, |q| as uint8; |-128| = 128
-      const uint32_t b = __byte_perm(a, 0, 0x2301);     // partner of each byte
-      const uint32_t mx = __vmaxu4(a, b), mn = __vminu4(a, b);
-      const uint32_t m = (mx & 0x00ff00ffu) + ((mn >> 1) & 0x007f007fu);  // two magnitudes <= 192
-      part += (m & 0xffffu) + (m >> 16);
-    }
-    sum += part;
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(FULL, sum, o);
   __shared__ unsigned long long s_part[4];
-  if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = sum;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned long long total = s_part[0] + s_part[1] + s_part[2] + s_part[3];
-    const uint32_t n = (uint32_t)(q.n_bytes / 2);
-    const uint32_t mag = (uint32_t)(total / n);
-    const uint32_t idx = mag > 127u ? 127u : mag;
-    int32_t db = q.db_table[idx] - 42;
-    db -= (int32_t)q.gain_db[ch];
-    const bool present = db >= q.threshold[ch];
-    const bool tracking = q.tracking[ch] != 0;
-    q.allowed[ch] = (present || tracking) ? 1 : 0;  // START / PRESENT / END-of-signal tail
-    q.tracking[ch] = present ? 1 : 0;
-    q.magnitude[ch] = mag;
+  uint32_t k = 0;
+  for (uint64_t off = 0; off < q.n_bytes; off += q.block_bytes, ++k) {
+    const uint64_t len = q.n_bytes - off < q.block_bytes ? q.n_bytes - off : q.block_bytes;
+    unsigned long long sum = 0;
+    for (uint64_t c = threadIdx.x; c < len / 16; c += blockDim.x) {
+      const u32x4 v = ld_stream_u4(src + off + 16 * c);
+      const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+      uint32_t part = 0;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const uint32_t a = __vabs4(w[i] ^ flip);          // |i|, |q| as uint8; |-128| = 128
+        const uint32_t b = __byte_perm(a, 0, 0x2301);     // partner of each byte
+        const uint32_t mx = __vmaxu4(a, b), mn = __vminu4(a, b);
+        const uint32_t m = (mx & 0x00ff00ffu) + ((mn >> 1) & 0x007f007fu);  // two magnitudes <= 192
+        part += (m & 0xffffu) + (m >> 16);
+      }
+      sum += part;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(FULL, sum, o);
+    if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = sum;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      const unsigned long long total = s_part[0] + s_part[1] + s_part[2] + s_part[3];
+      const uint32_t n = (uint32_t)(len / 2);
+      const uint32_t mag = (uint32_t)(total / n);
+      const uint32_t idx = mag > 127u ? 127u : mag;
+      int32_t db = q.db_table[idx] - 42;
+      db -= (int32_t)q.gain_db[ch];
+      const bool present = db >= q.threshold[ch];
+      const bool tracking = q.tracking[ch] != 0;
+      const size_t at = (size_t)k * q.n_channels + ch;
+      q.allowed[at] = (present || tracking) ? 1 : 0;  // START / PRESENT / END-of-signal tail
+      q.tracking[ch] = present ? 1 : 0;
+      q.magnitude[at] = mag;
+    }
+    __syncthreads();  // s_part is written again by the next block
+  }
+}
+
+// ---------------------------------------------------------------------------
+// PCM compaction after a call demodulated in block passes: block k's samples were written at
+// column k * block_samples; the open blocks' samples move to the front of the row, in block
+// order. One CTA per channel. A block moves only when an earlier block was closed, so its
+// destination ends at or before its source starts; the blocks move one after the other, so a
+// later block's destination (which may lie in an earlier block's source) is written only once
+// that source has been read.
+// ---------------------------------------------------------------------------
+struct CompactParams {
+  int16_t *pcm;               // [n_channels][pcm_stride]
+  uint64_t pcm_stride;        // int16 elements between channels (a multiple of 8)
+  const uint8_t *allowed;     // [n_blocks][n_channels] gates of the call
+  uint32_t n_channels;
+  uint32_t n_blocks;
+  uint32_t block_samples;     // PCM samples of a full block (a multiple of 32)
+  uint32_t last_samples;      // PCM samples of the last block (any count)
+};
+
+__global__ void __launch_bounds__(256) pcm_compact_kernel(const CompactParams p) {
+  const uint32_t ch = blockIdx.x;
+  int16_t *row = p.pcm + (uint64_t)ch * p.pcm_stride;
+  uint4 *row8 = reinterpret_cast<uint4 *>(row);  // 8 samples per uint4
+  uint32_t dst = 0;  // a multiple of 32: every block before the last is block_samples long
+  for (uint32_t k = 0; k < p.n_blocks; ++k) {
+    if (!p.allowed[(size_t)k * p.n_channels + ch]) continue;
+    const uint32_t len = k + 1 == p.n_blocks ? p.last_samples : p.block_samples;
+    const uint32_t src = k * p.block_samples;
+    if (dst != src) {  // uniform over the CTA
+      for (uint32_t i = threadIdx.x; i < len / 8; i += blockDim.x) row8[dst / 8 + i] = row8[src / 8 + i];
+      for (uint32_t i = len / 8 * 8 + threadIdx.x; i < len; i += blockDim.x) row[dst + i] = row[src + i];
+      __syncthreads();
+    }
+    dst += len;
   }
 }
 

@@ -4,7 +4,7 @@
 // radios. No Python, no torch: this is what a C++ host links.
 //
 //   b200_bank [-n channels] [-g gpus] [-m am|fm|wbfm|ssb|mixed] [-b block_bytes] [-t ticks] [-s slots]
-//             [-q squelch_dbfs] [-i k]
+//             [-q squelch_dbfs] [-i k] [-k squelch_block_bytes]
 //
 // A tick is one block of every channel. The producer writes each tick in place into the bank's
 // pinned tick array (here: synthetic offset-binary IQ, a noisy carrier per channel); the bank
@@ -15,7 +15,9 @@
 // tick then hands back its gate and mean magnitude per radio, what the reference's signal-state and
 // signal-magnitude callbacks receive (IqDataProcessor.cc:771-790); the JSON line adds the open
 // (radio, tick) pairs and the mean magnitude. -i k dumps the IQ of every k-th radio
-// (IqDataProcessor.cc:756-760); the JSON line adds the dumped bytes.
+// (IqDataProcessor.cc:756-760); the JSON line adds the dumped bytes. -k sets the squelch block on
+// every shard (the reference's acceptIqData length, 32768 in Radio.cc): each tick is then gated
+// block by block, and with -q the JSON line adds open_blocks, the open (radio, block) pairs.
 #include <chrono>
 #include <cmath>
 #include <cstdint>
@@ -35,7 +37,7 @@ static int die(const char *what, sdr_bank *b)
 int main(int argc, char **argv)
 {
   uint32_t nChannels = 8192, nGpus = 1, ticks = 20, slots = 3, dumpEvery = 0;
-  uint64_t blockBytes = 32768;
+  uint64_t blockBytes = 32768, squelchBlock = 0;
   const char *mode = "mixed";
   bool squelch = false;
   int32_t squelchDbfs = -200;
@@ -50,6 +52,7 @@ int main(int argc, char **argv)
     else if (!strcmp(argv[i], "-s")) slots = (uint32_t)atol(argv[i + 1]);
     else if (!strcmp(argv[i], "-q")) { squelch = true; squelchDbfs = (int32_t)atol(argv[i + 1]); }
     else if (!strcmp(argv[i], "-i")) dumpEvery = (uint32_t)atol(argv[i + 1]);
+    else if (!strcmp(argv[i], "-k")) squelchBlock = (uint64_t)atol(argv[i + 1]);
   } // for
 
   std::vector<int> devices(nGpus);
@@ -75,6 +78,8 @@ int main(int argc, char **argv)
       if (sdr_bank_set_squelch_threshold(bank, ch, squelchDbfs)) return die("sdr_bank_set_squelch_threshold", bank);
     if (sdr_bank_enable_signal_reports(bank, 1)) return die("sdr_bank_enable_signal_reports", bank);
   } // if
+  if (squelchBlock && sdr_bank_set_squelch_block_bytes(bank, squelchBlock))
+    return die("sdr_bank_set_squelch_block_bytes", bank);
   // IqDataProcessor::enableIqDump on every k-th radio (IqDataProcessor.cc:633-669)
   if (dumpEvery)
     for (uint32_t ch = 0; ch < nChannels; ch += dumpEvery)
@@ -105,7 +110,7 @@ int main(int argc, char **argv)
 
   // the timed loop: commit a tick, retire the one two ticks back (radioApp.cc:103-111 is the sink)
   long long checksum = 0;
-  unsigned long long openChannelTicks = 0, dumpBytes = 0;
+  unsigned long long openChannelTicks = 0, openBlocks = 0, dumpBytes = 0;
   double magnitudeSum = 0;
   const uint32_t inFlight = slots - 1;
   const std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
@@ -135,6 +140,11 @@ int main(int argc, char **argv)
           openChannelTicks += allowed[ch];
           magnitudeSum += magnitude[ch];
         } // for
+        // every block's signal state, in block order (the reference's callbacks once per block)
+        uint32_t nBlocks;
+        if (sdr_bank_retired_signal_blocks(bank, &allowed, &magnitude, &nBlocks))
+          return die("sdr_bank_retired_signal_blocks", bank);
+        for (size_t i = 0; i < (size_t)nBlocks * nChannels; i++) openBlocks += allowed[i];
       } // if
       if (dumpEvery)
       {
@@ -156,8 +166,9 @@ int main(int argc, char **argv)
          nGpus, nChannels, mode, (unsigned long long)blockBytes, ticks, secs, samples / secs / 1e6,
          samples * 2.0 / secs / 1e9, checksum);
   if (squelch)
-    printf(", \"squelch_dbfs\": %d, \"open_channel_ticks\": %llu, \"mean_magnitude\": %.3f", (int)squelchDbfs,
-           openChannelTicks, magnitudeSum / ((double)ticks * nChannels));
+    printf(", \"squelch_dbfs\": %d, \"open_channel_ticks\": %llu, \"open_blocks\": %llu, \"mean_magnitude\": %.3f",
+           (int)squelchDbfs, openChannelTicks, openBlocks, magnitudeSum / ((double)ticks * nChannels));
+  if (squelchBlock) printf(", \"squelch_block_bytes\": %llu", (unsigned long long)squelchBlock);
   if (dumpEvery) printf(", \"dump_every\": %u, \"dump_bytes\": %llu", dumpEvery, dumpBytes);
   printf("}\n");
   sdr_bank_destroy(bank);
